@@ -17,6 +17,10 @@ value = n_total * K * (m+1) / seconds  [chain-steps/s].
 host cores.  Its step is a BOUNDED SAMPLE of the cycle (a few MALA+FM iterations + one flow-MH+FM iteration on a small
 ensemble); the line says what ran (`config.chains_total`, `sample`) and that the cycle rate is composed from the two
 measured phase times (`extrapolated: true`).  The `cpu_baseline` object of the default run is ONE such step.
+
+`--dump-outputs DIR` writes what the last timed step handed its caller (chain state, step info, FM loss, updated MLP
+parameters) to DIR/<name>.npy in float32, so that two builds can be compared output for output on identical inputs:
+every input of a run is a fixed function of the arguments (seeded fixture, seeded keys).  See dump_outputs().
 """
 from __future__ import annotations
 
@@ -71,7 +75,13 @@ def parse():
                         "one extra flow-MH iteration is then run untimed)")
     p.add_argument("--no_cpu_baseline", action="store_true")
     p.add_argument("--no_e2e", action="store_true")
+    p.add_argument("--dump-outputs", dest="dump_outputs", type=str, default=None, metavar="DIR",
+                   help="write the outputs of the last timed step to DIR/<name>.npy (float32, a fixed sample of large arrays)")
     a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        p.error("--dump-outputs applies to --impl b200")
     c = CONFIGS[a.config]
     a.chains = a.chains or c["n"]
     a.m = a.m if a.m is not None else c["m"]
@@ -305,6 +315,53 @@ def device_dist(cfg, dev):
     return Dm.GaussianMixture(ot.modes, ot.covs, ot.weights, device=dev)
 
 
+DUMP_ROWS, DUMP_PARAMS, DUMP_BYTES = 2048, 1 << 20, 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, loop, loss, n_total, off, world, rank):
+    """--dump-outputs: what the last timed step returned to its caller, as float32 DIR/<name>.npy.
+
+    The new chain state (position, logdensity, logdensity_grad), the step's info (acceptance_rate, is_accepted as 0/1,
+    proposed_position, proposed_weight), the FM loss of its update and the updated flat MLP parameter vector.  Per-chain
+    vectors hold every chain.  [chain, d] arrays hold the rows of DUMP_ROWS chains and `params` DUMP_PARAMS entries, both
+    drawn once by numpy seed 0 (sorted, all of them when there are fewer), which keeps the files under DUMP_BYTES at every
+    configuration.  Collective when chains are sharded over several ranks; rank 0 writes."""
+    import torch
+    import torch.distributed as tdist
+    dev = loop.states.position.device
+    n = loop.n
+
+    def sample(total, k):
+        idx = np.arange(total) if total <= k else np.sort(np.random.default_rng(0).choice(total, k, replace=False))
+        return torch.from_numpy(idx).to(dev)
+
+    def chains(t, idx):
+        # rows `idx` (global chain indices) of a per-chain array: each rank fills the rows of its shard, the others are
+        # zero, so the SUM all-reduce is a copy
+        out = torch.zeros((idx.numel(),) + tuple(t.shape[1:]), dtype=torch.float32, device=dev)
+        own = (idx >= off) & (idx < off + n)
+        out[own] = t[idx[own] - off].float()
+        if world > 1:
+            tdist.all_reduce(out)
+        return out.cpu().numpy()
+
+    rows, every = sample(n_total, DUMP_ROWS), torch.arange(n_total, device=dev)
+    st, info = loop.states, loop.last_info
+    flat = loop.P.flat
+    arrays = {"position": chains(st.position, rows), "logdensity": chains(st.logdensity, every),
+              "logdensity_grad": chains(st.logdensity_grad, rows),
+              "acceptance_rate": chains(info.acceptance_rate, every), "is_accepted": chains(info.is_accepted, every),
+              "proposed_position": chains(info.proposed_position, rows), "proposed_weight": chains(info.proposed_weight, every),
+              "loss": loss.detach().float().reshape(-1).cpu().numpy(),
+              "params": flat[sample(flat.numel(), DUMP_PARAMS)].float().cpu().numpy()}
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs would write {total} bytes"
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for name, v in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), v)
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     a = parse()
@@ -367,9 +424,10 @@ def main():
         torch.cuda.synchronize()
 
     def run_cycle():
-        # iterations count+1 .. count+cyc with exactly one flow-MH iteration (count % (m+1) == 0)
+        # iterations count+1 .. count+cyc with exactly one flow-MH iteration (count % (m+1) == 0); returns the last loss
         for _ in range(cyc):
-            loop.iteration()
+            loss = loop.iteration()
+        return loss
 
     # ---- warm-up -------------------------------------------------------------------------------
     if a.warmup_unit == "cycle":
@@ -395,7 +453,7 @@ def main():
     sync()
     e0.record()
     for _ in range(a.steps):
-        run_cycle()
+        last_loss = run_cycle()
         flow_stats.append(loop.gen.last_stats.get("ode"))
     loop.flush()                          # multi-rank runs pipeline the last AdamW update: it belongs to the timed work
     e1.record()
@@ -412,6 +470,8 @@ def main():
     stats_l = [s.cpu() for s in flow_stats if s is not None]
     ode_stats = stats_l[-1][:4].tolist() if stats_l else None
     chain_evals = [int(s[4:6].view(torch.int64).item()) for s in stats_l]          # rows ACTUALLY evaluated (compaction), per step
+    if a.dump_outputs:                    # before the phase timings below move the chains on
+        dump_outputs(a.dump_outputs, loop, last_loss, n_total, off, world, rank)
 
     # ---- per-phase timing (MALA iteration, FM update, flow iteration) for the roofline ------------
     def timed(fn, reps):
