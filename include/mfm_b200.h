@@ -74,14 +74,28 @@ typedef struct mfm_field {
     long long n_params;      /* total floats */
     const float* omega;      /* [F] fourier_random (module attribute, :350-351) */
     float grad_clip;         /* <=0: no clip; else clip grad logprob to +-grad_clip (:87-90) */
-    /* reference (base) distribution of the flow, ref_dists[args.ref_dist] (exe_flow_matching.py:48-54,149,244):
-     * IndepGaussian(dim, mean, var = ref_std^2); stdgauss = (0, 1), widegauss = (0, sqrt(5)).  Used by the conditional
-     * FM batch (x0 = mean + std * normal, :156) and by the independent / importance-sampling flow steps (:249-256,283-289). */
+    /* reference (base) distribution of the flow, ref_dists[args.ref_dist] (exe_flow_matching.py:48-54,149,244).  Used by the
+     * conditional FM batch (x0 = ref.sample_model, :156), by the independent / importance-sampling flow steps (:249-256,283-289)
+     * and by mfm_ref_sample / mfm_ref_logprob.  Kind ref_kind below; MFM_REF_INDEP_GAUSS: IndepGaussian(dim, mean,
+     * var = ref_std^2), stdgauss = (0, 1), widegauss = (0, sqrt(5)). */
     float ref_mean, ref_std;
     /* activation of the six hidden layers, args.non_linearity (exe_flow_matching.py:40-46, multi_modal.py:181):
      * MFM_ACT_RELU (0, the default of every configuration), TANH, ELU, GELU (jax.nn.gelu's default tanh approximation), SWISH */
     int act;
+    /* MFM_REF_INDEP_GAUSS (0): the IndepGaussian above (ref_log_norm, ref_band unused; a zero-filled tail is exactly that).
+     * MFM_REF_PHI4_BASE (1): PhiFourBase(dim, alpha, beta), prior_type 'coupled' (distributions.py:168-226), the Gaussian
+     * N(0, P^-1) with the tridiagonal precision P = beta (diag(2c + 1/c) - c (sub + super diagonal)), c = alpha dim.  P = L L^T with
+     * L lower bidiagonal (diagonal l, sub-diagonal s_i = L[i][i-1]); ref_band (device, 2 d + 2 floats) = a[d] (a_i = -s_{i+1} / l_i,
+     * a_{d-1} = 0), rl[d] (rl_i = 1 / l_i), beta c, beta / c.  sample_model = L^-T z, z = normal(key, (d,)), by the back-substitution
+     * x_{d-1} = rl_{d-1} z_{d-1}, x_i = a_i x_{i+1} + rl_i z_i; logprob(x) = -q/2 + ref_log_norm
+     * with q = beta (c sum_{i=0..d} (x_i - x_{i-1})^2 + sum x_i^2 / c), x_{-1} = x_d = 0, ref_log_norm = -d/2 log 2 pi + sum log l_i.
+     * d <= MFM_REF_BAND_MAX_DIM for this kind (the row is staged in shared memory). */
+    int ref_kind;
+    float ref_log_norm;
+    const float* ref_band;
 } mfm_field_t;
+enum { MFM_REF_INDEP_GAUSS = 0, MFM_REF_PHI4_BASE = 1 };
+#define MFM_REF_BAND_MAX_DIM 12192
 
 typedef struct mfm_ode_opts {
     float rtol, atol;        /* multi_modal.py:205-206 */
@@ -246,6 +260,12 @@ int mfm_flow_cis_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode
                       int per_chain_keys, int n, int chain_offset, int n_total, float* position, float* logdensity,
                       float* acceptance_rate, uint8_t* is_accepted, float* proposed_position, float* proposed_weight, int* stats,
                       void* ws, size_t ws_bytes, mfm_stream_t stream);
+
+/* ---- reference distribution of the flow (f->ref_kind; only the ref_* fields and dim of `f` are read) ------------------
+ * mfm_ref_sample: vmap(ref_dist.sample_model)(keys[n]) -> out [n,d] (exe_flow_matching.py:156,249,284,453).
+ * mfm_ref_logprob: vmap(ref_dist.logprob)(x[n,d]) -> out [n] (:251-252,283,289,457). */
+int mfm_ref_sample(const mfm_field_t* f, const uint32_t* keys, int n, float* out, mfm_stream_t stream);
+int mfm_ref_logprob(const mfm_field_t* f, int n, const float* x, float* out, mfm_stream_t stream);
 
 /* ---- flow-matching update (exe_flow_matching.py:151-179, 362-368, 129-137, 184) ------------- */
 size_t mfm_fm_workspace_bytes(const mfm_field_t* f, const mfm_target_t* t, int n);

@@ -37,6 +37,7 @@ class FieldDesc(C.Structure):
         ("params", c_f32p), ("w_off", C.c_longlong * 8), ("b_off", C.c_longlong * 8),
         ("n_params", C.c_longlong), ("omega", c_f32p), ("grad_clip", C.c_float),
         ("ref_mean", C.c_float), ("ref_std", C.c_float), ("act", C.c_int),
+        ("ref_kind", C.c_int), ("ref_log_norm", C.c_float), ("ref_band", c_f32p),
     ]
 
 
@@ -47,6 +48,8 @@ class OdeOpts(C.Structure):
 
 TARGET_GMM, TARGET_PHI4, TARGET_PINES, TARGET_GAUSS, TARGET_PINES_WHITE = 0, 1, 2, 3, 4
 ACTIVATIONS = {"relu": 0, "tanh": 1, "elu": 2, "gelu": 3, "swish": 4}
+REF_INDEP_GAUSS, REF_PHI4_BASE = 0, 1
+REF_BAND_MAX_DIM = 12192
 FLOW_RW_MH, FLOW_INDEP_MH = 0, 1
 
 _PT, _FP, _OP = C.POINTER(TargetDesc), C.POINTER(FieldDesc), C.POINTER(OdeOpts)
@@ -109,6 +112,8 @@ SIGNATURES = {
     "mfm_flow_cis_workspace_bytes": (C.c_size_t, [_FP, _PT, _OP, C.c_int, C.c_int]),
     "mfm_flow_cis_step": (C.c_int, [_FP, _PT, _OP, C.c_int, c_u32p, C.c_int, C.c_int, C.c_int, C.c_int, c_f32p, c_f32p,
                                     c_f32p, c_u8p, c_f32p, c_f32p, c_i32p, C.c_void_p, C.c_size_t, _S]),
+    "mfm_ref_sample": (C.c_int, [_FP, c_u32p, C.c_int, c_f32p, _S]),
+    "mfm_ref_logprob": (C.c_int, [_FP, C.c_int, c_f32p, c_f32p, _S]),
     "mfm_fm_workspace_bytes": (C.c_size_t, [_FP, _PT, C.c_int]),
     "mfm_fm_loss_grad": (C.c_int, [_FP, _PT, c_u32p, C.c_int, C.c_int, C.c_int, C.c_float, c_f32p, c_f32p, c_f32p,
                                    C.c_void_p, C.c_size_t, _S]),

@@ -16,6 +16,7 @@
 #include <string.h>
 #include <stdlib.h>
 #include "gemm_tf32x3.cuh"
+#include "ref_dist.cuh"
 
 namespace mfm {
 
@@ -1210,6 +1211,67 @@ __global__ void gauss_logprob_kernel(int n, int d, const float* __restrict__ x, 
     if (lane == 0) out[c] = s;
 }
 
+// PhiFourBase sample (ref_dist.sample_model with ref_kind MFM_REF_PHI4_BASE): out = L^-T z row by row, one warp per row (ref_dist.cuh);
+// z and out may alias.  Dynamic shared memory: band_row_floats(d) floats per warp.
+__global__ void __launch_bounds__(256)
+ref_band_solve_kernel(int n, int d, const float* __restrict__ band, const float* z, float* out) {
+    extern __shared__ float band_rows[];
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (c >= n) return;
+    const int m = (d + 31) >> 5, mp = m | 1;
+    const float inv_m = 1.0f / (float)m;
+    float* r = band_rows + (threadIdx.x >> 5) * 32 * mp;
+    for (int j = lane; j < d; j += 32) r[band_slot(j, m, mp, inv_m)] = z[(long long)c * d + j];
+    band_solve_warp(r, d, band, lane);
+    for (int j = lane; j < d; j += 32) out[(long long)c * d + j] = r[band_slot(j, m, mp, inv_m)];
+}
+
+// PhiFourBase log-density (ref_dist.logprob, distributions.py:168-226) in the sum-of-squares form, which has no cancellation:
+// -q/2 + log_norm, q = beta c sum_{i=0..d} (x_i - x_{i-1})^2 + (beta / c) sum x_i^2 with x_{-1} = x_d = 0; band[2d] = beta c,
+// band[2d + 1] = beta / c.  One warp per row.
+__global__ void __launch_bounds__(256)
+ref_band_logprob_kernel(int n, int d, const float* __restrict__ band, float log_norm, const float* __restrict__ x, float* __restrict__ out) {
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (c >= n) return;
+    const float w_diff = __ldg(band + 2 * d), w_sq = __ldg(band + 2 * d + 1);
+    const float* row = x + (long long)c * d;
+    float s = 0.0f;
+    for (int i = lane; i < d; i += 32) {
+        const float xi = row[i];
+        const float df = xi - (i > 0 ? row[i - 1] : 0.0f);
+        s = fmaf(w_diff, df * df, fmaf(w_sq, xi * xi, s));
+    }
+    if (lane == 0) { const float xl = row[d - 1]; s = fmaf(w_diff, xl * xl, s); }     // (x_d - x_{d-1})^2
+    s = warp_sum(s);
+    if (lane == 0) out[c] = fmaf(-0.5f, s, log_norm);
+}
+
+// z [n, d] standard normal rows -> reference samples out (may alias z): ref_sample_kernel for IndepGaussian, the band solve for
+// PhiFourBase.  One launch either way.
+static int ref_transform_rows(const mfm_field_t& f, int n, const float* z, float* out, cudaStream_t stream) {
+    const int d = f.dim;
+    if (f.ref_kind == MFM_REF_PHI4_BASE) {
+        const int wpb = band_warps_per_block(d);
+        ref_band_solve_kernel<<<ceil_div(n, wpb), 32 * wpb, (size_t)wpb * band_row_floats(d) * sizeof(float), stream>>>(n, d, f.ref_band, z, out);
+    } else {
+        const long long tot = (long long)n * d;
+        ref_sample_kernel<<<ceil_div(tot, 256), 256, 0, stream>>>(tot, f.ref_mean, f.ref_std, z, out);
+    }
+    MFM_LAUNCH_CHECK();
+    return MFM_OK;
+}
+// out[c] = ref_dist.logprob(x[c]); one launch
+static int ref_logprob_rows(const mfm_field_t& f, int n, const float* x, float* out, cudaStream_t stream) {
+    if (f.ref_kind == MFM_REF_PHI4_BASE)
+        ref_band_logprob_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, f.dim, f.ref_band, f.ref_log_norm, x, out);
+    else
+        gauss_logprob_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, f.dim, x, f.ref_mean, f.ref_std, out);
+    MFM_LAUNCH_CHECK();
+    return MFM_OK;
+}
+
 struct FlowAcceptArgs {
     int variant;
     const float *xp, *lp, *gp, *Vp, *V0, *logq_up, *logq_u0;
@@ -1328,8 +1390,7 @@ static int check_field(const mfm_field_t* f, const mfm_target_t* t, const mfm_od
     if (f->dim != t->dim) { mfm_set_last_error_msg("field.dim != target.dim"); return MFM_ERR_ARG; }
     if (f->hidden <= 0 || f->fourier_dim <= 0 || !f->params || !f->omega) { mfm_set_last_error_msg("bad field descriptor"); return MFM_ERR_ARG; }
     if (f->act < MFM_ACT_RELU || f->act > MFM_ACT_SWISH) { mfm_set_last_error_msg("unknown activation (mfm_field_t::act)"); return MFM_ERR_ARG; }
-    if (!(f->ref_std > 0.0f)) { mfm_set_last_error_msg("field.ref_std must be > 0 (reference distribution IndepGaussian(mean, std^2))"); return MFM_ERR_ARG; }
-    return MFM_OK;
+    return ref_check(f, false);
 }
 
 void mfm_debug_set_ode_small(int v) { g_ode_small = v ? 1 : 0; }      // test hook (not in the ABI header): fused small-shape solve on / off
@@ -1399,6 +1460,7 @@ int mfm_flow_mh_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_
     if (!rng_key || !position || !logdensity || !logdensity_grad) { mfm_set_last_error_msg("null argument"); return MFM_ERR_ARG; }
     if (n <= 0) return MFM_OK;
     if (variant != MFM_FLOW_RW_MH && variant != MFM_FLOW_INDEP_MH) { mfm_set_last_error_msg("unknown flow-MH variant"); return MFM_ERR_ARG; }
+    if (variant == MFM_FLOW_INDEP_MH && (rc = ref_check(f, true))) return rc;
     if (per_chain_keys) { chain_offset = 0; n_total = 0; }
     else if (n_total < chain_offset + n || chain_offset < 0) { mfm_set_last_error_msg("bad chain_offset/n_total"); return MFM_ERR_ARG; }
     const int d = f->dim;
@@ -1433,17 +1495,14 @@ int mfm_flow_mh_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_
         if (hutch && (rc = mfm_threefry_normal_batched(kh1, n, d, z, stream))) return rc;
         if ((rc = ode_solve(*f, *t, *o, +1, n, hutch ? z : nullptr, up, xp, Vp, stats, 1, S, B, zc, stream))) return rc;
     } else {
-        // independent proposal from the reference distribution IndepGaussian(mean, std^2) (:48-49,249)
-        ref_sample_kernel<<<ceil_div(tot, 256), 256, 0, stream>>>(tot, f->ref_mean, f->ref_std, eps, up);
-        MFM_LAUNCH_CHECK();
+        // independent proposal from the reference distribution (:48-54,249)
+        if ((rc = ref_transform_rows(*f, n, eps, up, stream))) return rc;
         if (hutch && (rc = mfm_threefry_normal_batched(kh1, n, d, z, stream))) return rc;
         if ((rc = ode_solve(*f, *t, *o, +1, n, hutch ? z : nullptr, up, xp, Vp, stats, 0, S, B, zc, stream))) return rc;
         if (hutch && (rc = mfm_threefry_normal_batched(kh2, n, d, z, stream))) return rc;
         if ((rc = ode_solve(*f, *t, *o, -1, n, hutch ? z : nullptr, position, u0, V0, stats, 1, S, B, zc, stream))) return rc;
-        gauss_logprob_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, d, up, f->ref_mean, f->ref_std, lq_up);
-        MFM_LAUNCH_CHECK();
-        gauss_logprob_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, d, u0, f->ref_mean, f->ref_std, lq_u0);
-        MFM_LAUNCH_CHECK();
+        if ((rc = ref_logprob_rows(*f, n, up, lq_up, stream))) return rc;                   // (:251-252)
+        if ((rc = ref_logprob_rows(*f, n, u0, lq_u0, stream))) return rc;
     }
     if ((rc = target_value_and_grad(*t, n, xp, lp, gp, nullptr, wt, stream))) return rc;
     FlowAcceptArgs A{variant, xp, lp, gp, Vp, V0, lq_up, lq_u0, kacc, position, logdensity, logdensity_grad,
@@ -1468,6 +1527,7 @@ int mfm_flow_cis_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode
     if (rc) return rc;
     if (!rng_key || !position || !logdensity) { mfm_set_last_error_msg("null argument"); return MFM_ERR_ARG; }
     if (n_is <= 0) { mfm_set_last_error_msg("num_importance_samples must be > 0 for conditional importance sampling"); return MFM_ERR_ARG; }
+    if ((rc = ref_check(f, true))) return rc;
     if (n <= 0) return MFM_OK;
     if ((long long)n * n_is > 0x7FFFFFFFll) { mfm_set_last_error_msg("n * num_importance_samples too large"); return MFM_ERR_UNSUPPORTED; }
     if (per_chain_keys) { chain_offset = 0; n_total = 0; }
@@ -1495,21 +1555,38 @@ int mfm_flow_cis_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode
     // pull the current state back: its weight (:282-283)
     if (hutch && (rc = mfm_threefry_normal_batched(kprev, n, d, z, stream))) return rc;
     if ((rc = ode_solve(*f, *t, *o, -1, n, hutch ? z : nullptr, position, u_prev, vol_prev, stats, 0, S, B, zc, stream))) return rc;
-    gauss_logprob_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, d, u_prev, f->ref_mean, f->ref_std, lq_prev);
-    MFM_LAUNCH_CHECK();
+    if ((rc = ref_logprob_rows(*f, n, u_prev, lq_prev, stream))) return rc;
     // K fresh reference samples per chain, pushed forward with their own probe keys (:284-287)
     if ((rc = mfm_threefry_normal_batched(ksample, M, d, gscr, stream))) return rc;
-    ref_sample_kernel<<<ceil_div((long long)M * d, 256), 256, 0, stream>>>((long long)M * d, f->ref_mean, f->ref_std, gscr, refs);
-    MFM_LAUNCH_CHECK();
+    if ((rc = ref_transform_rows(*f, M, gscr, refs, stream))) return rc;
     if (hutch && (rc = mfm_threefry_normal_batched(khutch, M, d, z, stream))) return rc;
     if ((rc = ode_solve(*f, *t, *o, +1, M, hutch ? z : nullptr, refs, samples, vols, stats, 1, S, B, zc, stream))) return rc;
     if ((rc = target_value_and_grad(*t, M, samples, ld, gscr, nullptr, wt, stream))) return rc;      // logprob_beta of the samples (:288)
-    gauss_logprob_kernel<<<ceil_div(M, 8), 256, 0, stream>>>(M, d, refs, f->ref_mean, f->ref_std, lq);
-    MFM_LAUNCH_CHECK();
+    if ((rc = ref_logprob_rows(*f, M, refs, lq, stream))) return rc;
     CisArgs A{K, ld, lq, vols, lq_prev, vol_prev, samples, kchoice, wbuf, position, logdensity, acceptance_rate, proposed_position, proposed_weight, is_accepted, rng_x64()};
     cis_select_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(n, d, A);
     MFM_LAUNCH_CHECK();
     return MFM_OK;
+}
+
+int mfm_ref_sample(const mfm_field_t* f, const uint32_t* keys, int n, float* out, mfm_stream_t stream) {
+    if (!f) { mfm_set_last_error_msg("null descriptor"); return MFM_ERR_ARG; }
+    int rc = ref_check(f, true);
+    if (rc) return rc;
+    if (n <= 0) return MFM_OK;
+    if (!keys || !out || f->dim <= 0) { mfm_set_last_error_msg("null argument or dim <= 0 (mfm_ref_sample)"); return MFM_ERR_ARG; }
+    // normal(keys[c], (d,)) into out, then mean + std * z (exactly IndepGaussian.sample_model) or the band solve in place
+    if ((rc = mfm_threefry_normal_batched(keys, n, f->dim, out, stream))) return rc;
+    return ref_transform_rows(*f, n, out, out, stream);
+}
+
+int mfm_ref_logprob(const mfm_field_t* f, int n, const float* x, float* out, mfm_stream_t stream) {
+    if (!f) { mfm_set_last_error_msg("null descriptor"); return MFM_ERR_ARG; }
+    int rc = ref_check(f, false);
+    if (rc) return rc;
+    if (n <= 0) return MFM_OK;
+    if (!x || !out || f->dim <= 0) { mfm_set_last_error_msg("null argument or dim <= 0 (mfm_ref_logprob)"); return MFM_ERR_ARG; }
+    return ref_logprob_rows(*f, n, x, out, stream);
 }
 
 }  // extern "C"

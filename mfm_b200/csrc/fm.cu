@@ -8,6 +8,7 @@
 #include "internal.h"
 #include "gemm_tf32x3.cuh"
 #include "gemm_tcgen05_wgrad16.cuh"
+#include "ref_dist.cuh"
 
 namespace mfm {
 
@@ -61,6 +62,64 @@ fm_batch_kernel(const uint32_t* __restrict__ rng_key, int n, int chain_offset, i
     if (xt_amax) {
         amax_publish_warp(xt_amax, vm);                                    // x_t is the A operand of Dense_2 / the K^-1 GEMM
         amax_publish_warp(xt_amax + (AM_TGT - AM_X), tm);                  // (xt_amax is slot AM_X of the pool) bounds the loss gradient
+    }
+}
+
+// The same batch with the PhiFourBase reference distribution (ref_kind MFM_REF_PHI4_BASE): x0 = L^-T z where z is the normal row
+// fm_batch_kernel draws (same keys, same paired float32 layout, same x64 layout).  The row z is staged in shared memory
+// (band_solve_warp, ref_dist.cuh), solved there, and then x_t / target are formed exactly as above.  Dynamic shared memory:
+// band_row_floats(d) floats per warp.
+__global__ void __launch_bounds__(256)
+fm_batch_phi4_kernel(const uint32_t* __restrict__ rng_key, int n, int chain_offset, int n_total, int d, float sigma,
+                     const float* __restrict__ band, const float* __restrict__ x, float* __restrict__ times, float* __restrict__ xt,
+                     float* __restrict__ target, float* __restrict__ xt_amax, int x64) {
+    __shared__ double2 ltab[16];
+    extern __shared__ float band_rows[];
+    log_tab_load(ltab);                                                    // (before any warp leaves: contains a barrier)
+    const int lane = threadIdx.x & 31;
+    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (c >= n) return;                                                    // whole warps leave together
+    const int m = (d + 31) >> 5, mp = m | 1;
+    const float inv_m = 1.0f / (float)m;
+    float* r = band_rows + (threadIdx.x >> 5) * 32 * mp;
+    float vm = 0.0f, tm = 0.0f;
+    const uint32_t gc = (uint32_t)(chain_offset + c);
+    const u32x2 k_time = threefry_split_key(rng_key[0], rng_key[1], 0u, 4u);
+    const u32x2 k_ref = threefry_split_key(rng_key[0], rng_key[1], 1u, 4u);
+    const u32x2 k_gauss = threefry_split_key(rng_key[0], rng_key[1], 2u, 4u);
+    const float t = rng_uniform_at(k_time.a, k_time.b, gc, (uint32_t)n_total, x64);
+    const u32x2 k_row = threefry_split_key(k_ref.a, k_ref.b, gc, (uint32_t)n_total);
+    const uint32_t total = (uint32_t)n_total * (uint32_t)d;
+    const uint32_t half = ((uint32_t)d + 1u) >> 1;
+    // z = normal(k_row, (d,)) into shared memory
+    for (uint32_t b = lane; b < half; b += 32) {
+        const uint32_t hi = b + half;
+        const bool has_hi = hi < (uint32_t)d;
+        if (x64) {
+            r[band_slot((int)b, m, mp, inv_m)] = rng_normal_at(k_row.a, k_row.b, b, (uint32_t)d, 1);
+            if (has_hi) r[band_slot((int)hi, m, mp, inv_m)] = rng_normal_at(k_row.a, k_row.b, hi, (uint32_t)d, 1);
+        } else {
+            const u32x2 o = threefry2x32(k_row.a, k_row.b, b, has_hi ? hi : 0u);
+            r[band_slot((int)b, m, mp, inv_m)] = bits_to_normal_t(o.a, ltab);
+            if (has_hi) r[band_slot((int)hi, m, mp, inv_m)] = bits_to_normal_t(o.b, ltab);
+        }
+    }
+    band_solve_warp(r, d, band, lane);                                     // ref_dist.sample_model: x0 = L^-T z
+    const float omt = 1.0f - t;
+    for (int j = lane; j < d; j += 32) {
+        const float x0 = r[band_slot(j, m, mp, inv_m)];
+        const float eps = x64 ? rng_normal_at(k_gauss.a, k_gauss.b, gc * (uint32_t)d + j, total, 1) : rng_normal_at_t(k_gauss.a, k_gauss.b, gc * (uint32_t)d + j, total, ltab);
+        const long long idx = (long long)c * d + j;
+        const float xv = x[idx];
+        const float xtv = __fadd_rn(__fadd_rn(__fmul_rn(sigma, eps), __fmul_rn(t, xv)), __fmul_rn(omt, x0));   // (:167)
+        xt[idx] = xtv; vm = fmaxf(vm, fabsf(xtv));
+        const float tg = xv - x0;                                          // :168
+        target[idx] = tg; tm = fmaxf(tm, fabsf(tg));
+    }
+    if (lane == 0) times[c] = t;
+    if (xt_amax) {                                                         // the same maxima fm_batch_kernel publishes
+        amax_publish_warp(xt_amax, vm);
+        amax_publish_warp(xt_amax + (AM_TGT - AM_X), tm);
     }
 }
 
@@ -630,11 +689,11 @@ using namespace mfm;
 
 size_t mfm_fm_workspace_bytes(const mfm_field_t* f, const mfm_target_t* t, int n) { return fm_bytes(*f, *t, n); }
 
-static int fm_check(const mfm_field_t* f, const mfm_target_t* t) {
+// samples_ref: the call draws x0 from the reference distribution (the conditional batch)
+static int fm_check(const mfm_field_t* f, const mfm_target_t* t, bool samples_ref = false) {
     if (!f || !t) { mfm_set_last_error_msg("null descriptor"); return MFM_ERR_ARG; }
     if (f->dim != t->dim) { mfm_set_last_error_msg("field.dim != target.dim"); return MFM_ERR_ARG; }
-    if (!(f->ref_std > 0.0f)) { mfm_set_last_error_msg("field.ref_std must be > 0 (reference distribution IndepGaussian(mean, std^2))"); return MFM_ERR_ARG; }
-    return MFM_OK;
+    return ref_check(f, samples_ref);
 }
 
 int mfm_fm_loss_grad(const mfm_field_t* f, const mfm_target_t* t, const uint32_t* rng_key, int n, int chain_offset,
@@ -648,7 +707,7 @@ int mfm_fm_loss_grad_part(const mfm_field_t* f, const mfm_target_t* t, const uin
                           int n_total, float sigma, const float* positions, float* loss_out, float* grads, void* ws,
                           size_t ws_bytes, int part, mfm_stream_t stream) {
     mfm::CrossScope cross_scope;
-    int rc = fm_check(f, t);
+    int rc = fm_check(f, t, true);
     if (rc) return rc;
     if (part < 0 || part > 2) { mfm_set_last_error_msg("part must be 0, 1 or 2"); return MFM_ERR_ARG; }
     if (!rng_key || !positions || !loss_out || !grads) { mfm_set_last_error_msg("null argument"); return MFM_ERR_ARG; }
@@ -661,8 +720,14 @@ int mfm_fm_loss_grad_part(const mfm_field_t* f, const mfm_target_t* t, const uin
     float* xt_amax = (mfm::tc2h::gemm_h16() && M.B.amax) ? M.B.amax + AM_X : nullptr;
     if (part != 2) {
         if (M.B.amax) MFM_CUDA_CHECK(cudaMemsetAsync(M.B.amax + AM_EVAL_END, 0, (AM_POOL - AM_EVAL_END) * sizeof(float), stream));   // this pass's maxima
-        fm_batch_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(rng_key, n, chain_offset, n_total, f->dim, sigma, f->ref_mean, f->ref_std,
-                                                             positions, M.times, M.xt, M.target, xt_amax, rng_x64());
+        if (f->ref_kind == MFM_REF_PHI4_BASE) {
+            const int wpb = band_warps_per_block(f->dim);
+            fm_batch_phi4_kernel<<<ceil_div(n, wpb), 32 * wpb, (size_t)wpb * band_row_floats(f->dim) * sizeof(float), stream>>>(
+                rng_key, n, chain_offset, n_total, f->dim, sigma, f->ref_band, positions, M.times, M.xt, M.target, xt_amax, rng_x64());
+        } else {
+            fm_batch_kernel<<<ceil_div(n, 8), 256, 0, stream>>>(rng_key, n, chain_offset, n_total, f->dim, sigma, f->ref_mean, f->ref_std,
+                                                                 positions, M.times, M.xt, M.target, xt_amax, rng_x64());
+        }
         MFM_LAUNCH_CHECK();
     }
     return fm_forward_backward(*f, *t, n, M, loss_out, grads, stream, part, xt_amax, xt_amax != nullptr);   // fm_batch_kernel tracks max |target| too

@@ -12,7 +12,7 @@ void mfm_set_last_error(cudaError_t e, const char* file, int line) {
 }
 void mfm_set_last_error_msg(const char* msg) { snprintf(g_err, sizeof(g_err), "%s", msg); }
 extern "C" const char* mfm_last_error(void) { return g_err; }
-extern "C" int mfm_version(void) { return 100; }
+extern "C" int mfm_version(void) { return 101; }   // 101: mfm_field_t grew (ref_kind, ref_log_norm, ref_band)
 unsigned long long g_mfm_launches = 0;
 #include <stdlib.h>
 namespace mfm {

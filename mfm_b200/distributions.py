@@ -135,6 +135,95 @@ class IndepGaussian(Distribution):
         """rng_key uint32[2] -> [d]; uint32[N,2] -> [N,d] (the vmapped form, exe_flow_matching.py:155)."""
         return self.mean + self.std * mrandom.normal(rng_key, (self.dim,))
 
+    def _fill_ref(self, d: _lib.FieldDesc):
+        """As the reference distribution of a flow (mfm_field_t::ref_*)."""
+        d.ref_kind, d.ref_mean, d.ref_std = _lib.REF_INDEP_GAUSS, self.mean, self.std
+
+
+def phi_four_base_band(dim, alpha=0.1, beta=20.0):
+    """Band Cholesky factor of PhiFourBase's tridiagonal precision P = beta (diag(2c + 1/c) - c (sub + super diagonal)),
+    c = alpha dim, in float64: P = L L^T with L lower bidiagonal, diagonal l[d] and sub-diagonal s[d] (s[i] = L[i][i-1],
+    s[0] = 0).  Returns (l, s, log_norm) with log_norm = -d/2 log 2 pi + sum log l_i = -(d log 2 pi + log det P^-1) / 2, the
+    constant of logprob (distributions.py:168-226)."""
+    c = alpha * dim
+    p, q = beta * (2.0 * c + 1.0 / c), -beta * c
+    l, s = np.empty(dim), np.zeros(dim)
+    l[0] = np.sqrt(p)
+    for i in range(1, dim):
+        s[i] = q / l[i - 1]
+        l[i] = np.sqrt(p - s[i] * s[i])
+    log_norm = float(-0.5 * dim * np.log(2.0 * np.pi) + np.log(l).sum())
+    return l, s, log_norm
+
+
+class PhiFourBase(Distribution):
+    """distributions.py:168-226: the Gaussian part of the phi-four action, N(0, P^-1) with the tridiagonal precision P above;
+    ref_dists['phifour'] (exe_flow_matching.py:53).  A reference distribution only: sample_model = L^-T normal(key, (d,)) and
+    logprob run as CUDA kernels (mfm_ref_sample / mfm_ref_logprob, one band solve / one sum of squares per row, never a dense
+    d x d factor).  The band factor is formed in float64 here and handed to the device as float32."""
+
+    def __init__(self, dim, alpha=0.1, beta=20.0, prior_type="coupled", device=None):
+        if prior_type == "coupled_pbc":
+            raise NotImplementedError("prior_type='coupled_pbc' cannot be constructed in the reference: it assigns into jnp arrays "
+                                      "and divides dim to a float (distributions.py:168-226)")
+        if prior_type != "coupled":
+            raise ValueError(f"unknown prior_type {prior_type!r}: 'coupled'")
+        super().__init__(device)
+        self.dim, self.alpha, self.beta, self.prior_type = int(dim), float(alpha), float(beta), prior_type
+        c = self.alpha * self.dim
+        self.l, self.s, self.log_norm = phi_four_base_band(self.dim, self.alpha, self.beta)
+        # a[d] = -s_{i+1} / l_i, 1 / l[d], beta c, beta / c: the layout of mfm_field_t::ref_band (back-substitution coefficients
+        # x_i = a_i x_{i+1} + z_i / l_i, rounded to float32 once from float64)
+        a = np.zeros(self.dim)
+        a[:-1] = -self.s[1:] / self.l[:-1]
+        self.band = self._tensor(np.concatenate([a, 1.0 / self.l, [self.beta * c, self.beta / c]]))
+        self.can_sample = True
+
+    def _fill_ref(self, d: _lib.FieldDesc):
+        """As the reference distribution of a flow (mfm_field_t::ref_*).  ref_mean / ref_std stay (0, 1)."""
+        d.ref_mean, d.ref_std = 0.0, 1.0
+        d.ref_kind, d.ref_band, d.ref_log_norm = _lib.REF_PHI4_BASE, self.band.data_ptr(), self.log_norm
+
+    def _ref_desc(self) -> _lib.FieldDesc:
+        d = _lib.FieldDesc()
+        d.dim = self.dim
+        self._fill_ref(d)
+        return d
+
+    def _desc(self, beta: float):
+        raise NotImplementedError("PhiFourBase is a reference distribution only: it has no target descriptor (no MALA, no field "
+                                  "score term)")
+
+    def tempered(self, beta: float = 1.0):
+        raise NotImplementedError("PhiFourBase is a reference distribution only: it cannot be tempered or used as a MALA target")
+
+    def initialize_model(self, rng_key, n_chain):
+        raise NotImplementedError("PhiFourBase is a reference distribution only: it is not a target to initialise chains for")
+
+    def sample_model(self, rng_key):
+        """rng_key uint32[2] -> [d]; uint32[N,2] -> [N,d] (vmap(sample_model), exe_flow_matching.py:156,453)."""
+        lib = _lib.load()
+        single = rng_key.dim() == 1
+        keys = (rng_key[None] if single else rng_key).contiguous()
+        out = torch.empty((keys.shape[0], self.dim), dtype=torch.float32, device=keys.device)
+        _lib.check(lib.mfm_ref_sample(self._ref_desc(), _lib.ptr(keys), keys.shape[0], _lib.ptr(out), _lib.stream()))
+        return out[0] if single else out
+
+    def logprob(self, x):
+        """x [d] -> scalar; [N,d] -> [N]:  -x^T P x / 2 + log_norm."""
+        lib = _lib.load()
+        single = x.dim() == 1
+        xx = (x[None] if single else x).to(torch.float32).contiguous()
+        out = torch.empty(xx.shape[0], dtype=torch.float32, device=xx.device)
+        _lib.check(lib.mfm_ref_logprob(self._ref_desc(), xx.shape[0], _lib.ptr(xx), _lib.ptr(out), _lib.stream()))
+        return out[0] if single else out
+
+    def loglik(self, x):
+        return self.logprob(x)
+
+    def logprior(self, x):
+        return torch.zeros(x.shape[:-1], dtype=torch.float32, device=x.device)          # logprior is 0 (distributions.py:168-226)
+
 
 class PhiFour(Distribution):
     """distributions.py:114-165 (Dirichlet(0) boundary, no tilt)."""

@@ -22,7 +22,7 @@ import torch
 
 from . import _lib, parallel, random as mrandom
 from .bblackjax.mcmc.mala import MALAInfo, MALAState, init, mala_step
-from .distributions import DeviceLogDensity, Distribution, GaussianMixture, IndepGaussian
+from .distributions import DeviceLogDensity, Distribution, GaussianMixture, IndepGaussian, PhiFourBase
 
 logger = logging.getLogger(__name__)
 
@@ -33,11 +33,12 @@ def _broken_ref(name, why):
 
 
 # exe_flow_matching.py:48-54.  'bimodal' and 'flat' fail at construction in the reference as coded (GaussianMixture(dim)
-# indexes an int, FlatDistribution() misses its argument); they raise here too.  'phifour' (PhiFourBase, a dense Gaussian)
-# is a §8(f) "next" row.
+# indexes an int, FlatDistribution() misses its argument); they raise here too.  'phifour' is PhiFourBase(dim) with its defaults
+# (alpha 0.1, beta 20, prior_type 'coupled'), a Gaussian with a tridiagonal precision that the kernels apply through its band factor.
 ref_dists = {
     "stdgauss": lambda dim, device=None: IndepGaussian(dim, device=device),
     "widegauss": lambda dim, device=None: IndepGaussian(dim, var=5.0, device=device),
+    "phifour": lambda dim, device=None: PhiFourBase(dim, device=device),
     "bimodal": _broken_ref("bimodal", "GaussianMixture(dim) takes the modes, not a dimension (distributions.py:43-49)"),
     "flat": _broken_ref("flat", "FlatDistribution() is called without its dim argument (exe_flow_matching.py:52)"),
 }
@@ -46,7 +47,7 @@ ref_dists = {
 def make_ref_dist(args, dim, device=None):
     name = getattr(args, "ref_dist", "stdgauss")
     if name not in ref_dists:
-        raise NotImplementedError(f"ref_dist='{name}' is not implemented on device (stdgauss, widegauss are)")
+        raise NotImplementedError(f"ref_dist='{name}' is not implemented on device (stdgauss, widegauss, phifour are)")
     return ref_dists[name](dim, device=device)
 
 
@@ -127,13 +128,20 @@ class VectorFieldNet:
         self.fourier_random = fourier_random.to(torch.float32).contiguous()
         self.grad_clip = float(grad_clip) if grad_clip else 0.0
         self.ref_mean, self.ref_std = 0.0, 1.0     # reference distribution of the flow (set_ref_dist)
+        self.ref = None                            # None: IndepGaussian(ref_mean, ref_std^2)
 
-    def set_ref_dist(self, ref: IndepGaussian):
+    def set_ref_dist(self, ref):
         """ref_dists[args.ref_dist](dim) (:149,244): the kernels draw x0 / the independent proposal from it and evaluate
         its log-density, so its parameters travel in the field descriptor."""
-        if not isinstance(ref, IndepGaussian):
-            raise NotImplementedError("the device kernels implement IndepGaussian reference distributions (stdgauss, widegauss)")
-        self.ref_mean, self.ref_std = float(ref.mean), float(ref.std)
+        if isinstance(ref, IndepGaussian):
+            self.ref_mean, self.ref_std, self.ref = float(ref.mean), float(ref.std), None
+        elif isinstance(ref, PhiFourBase):
+            if ref.dim != self.dist.dim:
+                raise ValueError(f"reference distribution dim {ref.dim} != target dim {self.dist.dim}")
+            self.ref_mean, self.ref_std, self.ref = 0.0, 1.0, ref
+        else:
+            raise NotImplementedError("the device kernels implement the IndepGaussian (stdgauss, widegauss) and PhiFourBase "
+                                      "(phifour) reference distributions")
         return self
 
     def init(self, rng_key, x0=None, t0=None, head_scale: float = 0.0) -> VectorFieldParams:
@@ -159,6 +167,8 @@ class VectorFieldNet:
         d.grad_clip = self.grad_clip
         d.ref_mean, d.ref_std = self.ref_mean, self.ref_std
         d.act = self.act
+        if self.ref is not None:
+            self.ref._fill_ref(d)
         return d
 
     def apply(self, P: VectorFieldParams, x: torch.Tensor, t: torch.Tensor, z: Optional[torch.Tensor] = None,
