@@ -65,8 +65,14 @@ typedef struct mfm_target {
 
 /* VectorFieldNet parameters (exe_flow_matching.py:56-90).  One flat fp32 parameter buffer; layer i
  * (flax name Dense_i) has kernel [in_i, out_i] row-major at params + w_off[i] and bias [out_i] at
- * params + b_off[i].  Layers: 0,1 time branch (2F->H->H), 2,3 x branch (d->H->H), 4 nn_t head
- * (H->d), 5,6 joint (2H->H->H), 7 nn_xt head (H->d). */
+ * params + b_off[i].  Each branch has two hidden layers, hidden_t = [Ht0, Ht1], hidden_x = [Hx0, Hx1],
+ * hidden_xt = [Hxt0, Hxt1] (the fields at the end of the struct):
+ *   Dense_0 (2F, Ht0)   Dense_1 (Ht0, Ht1)          time branch -> s_t
+ *   Dense_2 (d, Hx0)    Dense_3 (Hx0, Hx1)          x branch    -> s_x
+ *   Dense_4 (Ht1, d)                                nn_t head
+ *   Dense_5 (Hx1 + Ht1, Hxt0), input [s_x | s_t]    Dense_6 (Hxt0, Hxt1)   joint branch
+ *   Dense_7 (Hxt1, d)                               nn_xt head
+ * With all six widths equal to `hidden` = H: 2F->H->H, d->H->H, H->d, 2H->H->H, H->d. */
 typedef struct mfm_field {
     int dim, hidden, fourier_dim;
     const float* params;     /* flat buffer */
@@ -93,6 +99,10 @@ typedef struct mfm_field {
     int ref_kind;
     float ref_log_norm;
     const float* ref_band;
+    /* hidden widths of the three branches (layer table above).  All six zero: every width is `hidden` (a zero-filled tail is
+     * the equal-width network).  Otherwise all six must be > 0 and `hidden` must equal the largest of them, else the field and
+     * FM entry points return MFM_ERR_ARG.  Only two layers per branch are supported. */
+    int hidden_t[2], hidden_x[2], hidden_xt[2];
 } mfm_field_t;
 enum { MFM_REF_INDEP_GAUSS = 0, MFM_REF_PHI4_BASE = 1 };
 #define MFM_REF_BAND_MAX_DIM 12192

@@ -38,6 +38,7 @@ class FieldDesc(C.Structure):
         ("n_params", C.c_longlong), ("omega", c_f32p), ("grad_clip", C.c_float),
         ("ref_mean", C.c_float), ("ref_std", C.c_float), ("act", C.c_int),
         ("ref_kind", C.c_int), ("ref_log_norm", C.c_float), ("ref_band", c_f32p),
+        ("hidden_t", C.c_int * 2), ("hidden_x", C.c_int * 2), ("hidden_xt", C.c_int * 2),
     ]
 
 

@@ -202,8 +202,9 @@ __global__ void __launch_bounds__(256) weight_norms_kernel(const float* __restri
 }
 
 static void layer_dims(const mfm_field_t& F, int i, int& in, int& out) {
-    const int d = F.dim, H = F.hidden, Fd = F.fourier_dim;
-    const int ins[8] = {2 * Fd, H, d, H, H, 2 * H, H, H}, outs[8] = {H, H, H, H, d, H, H, d};
+    const int d = F.dim, Fd = F.fourier_dim;
+    const FieldWidths W = field_widths(F);
+    const int ins[8] = {2 * Fd, W.t0, d, W.x0, W.t1, W.cat(), W.xt0, W.xt1}, outs[8] = {W.t0, W.t1, W.x0, W.x1, d, W.xt0, W.xt1, d};
     in = ins[i]; out = outs[i];
 }
 
@@ -441,45 +442,57 @@ __global__ void div_finish_kernel(int n, int n_tiles, const float* __restrict__ 
 // field evaluation
 // ---------------------------------------------------------------------------------------------
 size_t field_bufs_bytes(const mfm_field_t& F, const mfm_target_t& T, int n, bool hutch) {
-    const size_t H = F.hidden, d = F.dim, N = n;
-    size_t b = ws_slice(N * 2 * F.fourier_dim, 4) + ws_slice(N * H, 4) * 6 + ws_slice(N * 2 * H, 4) + ws_slice(N * d, 4) * 3;
-    if (hutch) b += ws_slice(N * H, 4) + ws_slice(N * d, 4) + ws_slice(N * gemm_n_tiles((int)d), 4);
-    else b += 2 * ws_slice(N * d * H, 4);
-    b += ws_slice(N * 2 * F.fourier_dim, 4) + ws_slice(N * H, 4) * 6 + ws_slice(N * 2 * H, 4);      // pre-split copies (ff, h0, h2, h5, h6, ta, tb, cat)
-    if (F.act != MFM_ACT_RELU) b += ws_slice(N * H, 4) * 4 + ws_slice(N * 2 * H, 4);                // activation derivatives
+    const FieldWidths W = field_widths(F);
+    const size_t d = F.dim, N = n, C = W.cat(), Tn = W.tan();
+    // h0, h2, h5, h6 and the tangent pair ta, tb (x and joint branches only)
+    const size_t acts = ws_slice(N * W.t0, 4) + ws_slice(N * W.x0, 4) + ws_slice(N * W.xt0, 4) + ws_slice(N * W.xt1, 4) + 2 * ws_slice(N * Tn, 4);
+    size_t b = ws_slice(N * 2 * F.fourier_dim, 4) + acts + ws_slice(N * C, 4) + ws_slice(N * d, 4) * 3;
+    if (hutch) b += ws_slice(N * W.x0, 4) + ws_slice(N * d, 4) + ws_slice(N * gemm_n_tiles((int)d), 4);
+    else b += 2 * ws_slice(N * d * Tn, 4);
+    b += ws_slice(N * 2 * F.fourier_dim, 4) + acts + ws_slice(N * C, 4);      // pre-split copies (ff, h0, h2, h5, h6, ta, tb, cat)
+    if (F.act != MFM_ACT_RELU)                                                // activation derivatives
+        b += ws_slice(N * W.t0, 4) + ws_slice(N * W.x0, 4) + ws_slice(N * W.xt0, 4) + ws_slice(N * W.xt1, 4) + ws_slice(N * C, 4);
     if (T.kind == MFM_TARGET_PINES_WHITE) b += 4 * ws_slice(N * d, 4);
     return b + 3 * ws_slice((size_t)F.n_params, 4) + ws_slice(AM_POOL, 4);
 }
 
+// Whether the network runs on the scaled-fp16 path (tracked maxima, operator norms, weight mirrors, pre-split hand-over): every
+// width at least h16_min_hidden() and, for a network with unequal widths, every width a multiple of 16 (then the s_t half of
+// cat's pre-split copy, at column x1, stays 64-byte aligned).  Otherwise its layers run on the kernels narrow networks use.
+static bool field_h16_widths(const FieldWidths& W) {
+    return W.narrowest() >= tc2h::h16_min_hidden() && (W.equal || W.all16());
+}
+
 bool field_bufs_take(FieldBufs& B, Workspace& w, const mfm_field_t& F, int n, bool hutch, const mfm_target_t* T) {
-    const size_t H = F.hidden, d = F.dim, N = n;
+    const FieldWidths W = field_widths(F);
+    const size_t d = F.dim, N = n, C = W.cat(), Tn = W.tan();
     B.ff = w.take<float>(N * 2 * F.fourier_dim);
-    B.h0 = w.take<float>(N * H); B.h2 = w.take<float>(N * H); B.h5 = w.take<float>(N * H); B.h6 = w.take<float>(N * H);
-    B.ta = w.take<float>(N * H); B.tb = w.take<float>(N * H);
-    B.cat = w.take<float>(N * 2 * H);
+    B.h0 = w.take<float>(N * W.t0); B.h2 = w.take<float>(N * W.x0); B.h5 = w.take<float>(N * W.xt0); B.h6 = w.take<float>(N * W.xt1);
+    B.ta = w.take<float>(N * Tn); B.tb = w.take<float>(N * Tn);
+    B.cat = w.take<float>(N * C);
     B.gt = w.take<float>(N * d); B.gc = w.take<float>(N * d); B.hx = w.take<float>(N * d);
     B.zw2 = B.zkinv = B.divpart = B.tan_a = B.tan_b = nullptr;
-    if (hutch) { B.zw2 = w.take<float>(N * H); B.zkinv = w.take<float>(N * d); B.divpart = w.take<float>(N * gemm_n_tiles((int)d)); }
-    else { B.tan_a = w.take<float>(N * d * H); B.tan_b = w.take<float>(N * d * H); }
+    if (hutch) { B.zw2 = w.take<float>(N * W.x0); B.zkinv = w.take<float>(N * d); B.divpart = w.take<float>(N * gemm_n_tiles((int)d)); }
+    else { B.tan_a = w.take<float>(N * d * Tn); B.tan_b = w.take<float>(N * d * Tn); }
     B.wt = w.take<float>((size_t)F.n_params);
     B.wx = w.take<float>((size_t)F.n_params); B.wxo = w.take<float>((size_t)F.n_params);
     B.amax = w.take<float>(AM_POOL);
     B.ff_s = w.take<float>(N * 2 * F.fourier_dim);
-    B.h0_s = w.take<float>(N * H); B.h2_s = w.take<float>(N * H); B.h5_s = w.take<float>(N * H); B.h6_s = w.take<float>(N * H);
-    B.ta_s = w.take<float>(N * H); B.tb_s = w.take<float>(N * H);
-    B.cat_s = w.take<float>(N * 2 * H);
+    B.h0_s = w.take<float>(N * W.t0); B.h2_s = w.take<float>(N * W.x0); B.h5_s = w.take<float>(N * W.xt0); B.h6_s = w.take<float>(N * W.xt1);
+    B.ta_s = w.take<float>(N * Tn); B.tb_s = w.take<float>(N * Tn);
+    B.cat_s = w.take<float>(N * C);
     B.dh0 = B.dh2 = B.dh5 = B.dh6 = B.dcat = nullptr;
     if (F.act != MFM_ACT_RELU) {
-        B.dh0 = w.take<float>(N * H); B.dh2 = w.take<float>(N * H); B.dh5 = w.take<float>(N * H); B.dh6 = w.take<float>(N * H);
-        B.dcat = w.take<float>(N * 2 * H);
+        B.dh0 = w.take<float>(N * W.t0); B.dh2 = w.take<float>(N * W.x0); B.dh5 = w.take<float>(N * W.xt0); B.dh6 = w.take<float>(N * W.xt1);
+        B.dcat = w.take<float>(N * C);
     }
     B.tscratch = nullptr;
     if (T && T->kind == MFM_TARGET_PINES_WHITE) { B.tscratch = w.take<float>(N * d); w.take<float>(N * d); w.take<float>(N * d); w.take<float>(N * d); }
     // fewer than 256 rows in every dense layer (tangent rows of the exact divergence included): nothing reaches the CTA-pair
     // tcgen05 kernel, so the per-call weight preparation for it (maximum, operator norms, two mirrors) and the maxima
     // bookkeeping are skipped altogether - at the small reference shapes they cost more than the layers themselves; the same for
-    // narrow networks (hidden < 512: memory-bound layers, see h16_min_hidden)
-    if (N * (hutch ? 1 : d) < 256 || (int)H < tc2h::h16_min_hidden()) {
+    // narrow networks (a width < 512: memory-bound layers, see h16_min_hidden) and unequal widths that are not multiples of 16
+    if (N * (hutch ? 1 : d) < 256 || !field_h16_widths(W)) {
         B.amax = nullptr; B.wx = B.wxo = nullptr;
         B.ff_s = B.h0_s = B.cat_s = B.h2_s = B.h5_s = B.h6_s = B.ta_s = B.tb_s = nullptr;
     }
@@ -493,7 +506,7 @@ bool field_bufs_take(FieldBufs& B, Workspace& w, const mfm_field_t& F, int n, bo
 // per-solve constants of the Hutchinson estimator: z W2 and (pines) z K^-1
 static int field_prepare_probe(const mfm_field_t& F, const mfm_target_t& T, int n, const float* z, FieldBufs& B, cudaStream_t st,
                                float z_bound) {
-    const int d = F.dim, H = F.hidden;
+    const int d = F.dim, H = field_widths(F).x0;      // z W2 has the width of Dense_2
     DenseAmax am; am.a_bound = z_bound;
     if (tc2h::gemm_h16() && B.amax) {       // exact max |z W2|: scales the gated tangent's pre-split copy in every field evaluation of the solve
         MFM_CUDA_CHECK(cudaMemsetAsync(B.amax + AM_ZW2, 0, sizeof(float), st));
@@ -514,7 +527,9 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
                const float* z, float sgn, float* out_v, float* out_l, FieldBufs& B, cudaStream_t st,
                const int* nr, const int* row_map, const float* x_amax, const float* x_split) {
     const float* zw2_amax = (tc2h::gemm_h16() && B.amax && z) ? B.amax + AM_ZW2 : nullptr;   // written by field_prepare_probe
-    const int d = F.dim, H = F.hidden, Fd = F.fourier_dim;
+    const int d = F.dim, Fd = F.fourier_dim;
+    const FieldWidths W = field_widths(F);
+    const int t0 = W.t0, t1 = W.t1, x0 = W.x0, x1 = W.x1, xt0 = W.xt0, xt1 = W.xt1, C = W.cat();
     int rc;
     // tensor maxima for the scaled-fp16 GEMMs (AmaxSlot): this evaluation's slots start from zero; x gets one reduction
     // when its producer did not track it (it feeds Dense_2 and, for pines, the K^-1 GEMM)
@@ -530,7 +545,7 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
     // pre-split copies: a layer's result leaves the epilogue in tensor-core format too (EpiStdS) and the consuming layer's TMA
     // loads that copy (no splitter work, a quarter less shared-memory traffic in the consumer)
     static const bool no_split = getenv("MFM_H16_NOSPLIT") != nullptr;      // debug: every layer splits its own A operand
-    const bool sp = !no_split && am != nullptr && B.h0_s != nullptr && H % 16 == 0 && (2 * Fd) % 16 == 0 && n >= 256 && ((reinterpret_cast<uintptr_t>(B.h0_s) | reinterpret_cast<uintptr_t>(B.cat_s)) & 63) == 0;
+    const bool sp = !no_split && am != nullptr && B.h0_s != nullptr && W.all16() && (2 * Fd) % 16 == 0 && n >= 256 && ((reinterpret_cast<uintptr_t>(B.h0_s) | reinterpret_cast<uintptr_t>(B.cat_s)) & 63) == 0;
     auto BD = [&](int i) -> float* { return am + AM_BOUND + i; };
     auto WC = [&](int l) -> const float* { return am + AM_WNORM_COL + l; };
     auto BA = [&](int l) -> const float* { return am + AM_BIAS + l; };
@@ -554,32 +569,32 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
     fourier_kernel<<<ceil_div((long long)n * Fd, 256), 256, 0, st>>>(n, Fd, F.omega, tfield, B.ff, nr, sp ? B.ff_s : nullptr, sp ? BD(AM_FF) : nullptr);
     MFM_LAUNCH_CHECK();
     // first layers of the two branches (the exact maxima of h0 and h2 feed the COMMON scale of cat = [s_x | s_t])
-    if ((rc = dense(n, 2 * Fd, H, B.ff, 2 * Fd, WT_(0), 2 * Fd, B_(0), act, B.h0, H, nullptr, 0, 1, st, nr,
-                    D_(OUT_(IN_(A_(nullptr, nullptr, 1.0f, slot(AM_H0)), B.ff_s, BD(AM_FF)), B.h0_s, AM_H0, 0, true), B.dh0, H)))) return rc;      // |cos|, |sin| <= 1
-    if ((rc = dense(n, d, H, x, d, WT_(2), d, B_(2), act, B.h2, H, nullptr, 0, 1, st, nr,
+    if ((rc = dense(n, 2 * Fd, t0, B.ff, 2 * Fd, WT_(0), 2 * Fd, B_(0), act, B.h0, t0, nullptr, 0, 1, st, nr,
+                    D_(OUT_(IN_(A_(nullptr, nullptr, 1.0f, slot(AM_H0)), B.ff_s, BD(AM_FF)), B.h0_s, AM_H0, 0, true), B.dh0, t0)))) return rc;      // |cos|, |sin| <= 1
+    if ((rc = dense(n, d, x0, x, d, WT_(2), d, B_(2), act, B.h2, x0, nullptr, 0, 1, st, nr,
                     D_(OUT_((x_split && x_amax) ? IN_(A_(x_amax, nullptr, 0, slot(AM_H2)), x_split, x_amax) : A_(x_amax, nullptr, 0, slot(AM_H2)),
-                            B.h2_s, AM_H2, 2, true), B.dh2, H)))) return rc;
-    {   // s_t and s_x: one scale for both halves of cat
-        DenseAmax mt = OUT_(IN_(A_(slot(AM_H0), nullptr, 0, slot(AM_ST)), B.h0_s, BD(AM_H0)), B.cat_s + H, AM_ST, 1, true);
+                            B.h2_s, AM_H2, 2, true), B.dh2, x0)))) return rc;
+    {   // s_t and s_x: one scale for both halves of cat = [s_x | s_t] (row stride x1 + t1, s_t from column x1)
+        DenseAmax mt = OUT_(IN_(A_(slot(AM_H0), nullptr, 0, slot(AM_ST)), B.h0_s, BD(AM_H0)), B.cat_s + x1, AM_ST, 1, true);
         // (h2's copy exists only when Dense_2 knew max |x|: dense() needs an input maximum to bound its output)
         DenseAmax mx = OUT_(A_(slot(AM_H2), nullptr, 0, slot(AM_SX)), B.cat_s, AM_SX, 3, true);
         if (x_amax) mx = IN_(mx, B.h2_s, BD(AM_H2));
         if (sp) { mt.alt_amax = slot(AM_H2); mt.alt_w_norm = WC(3); mt.alt_bias = BA(3); mx.alt_amax = slot(AM_H0); mx.alt_w_norm = WC(1); mx.alt_bias = BA(1); }
-        if ((rc = dense(n, H, H, B.h0, H, WT_(1), H, B_(1), act, B.cat + H, 2 * H, nullptr, 0, 1, st, nr, D_(mt, dmul ? B.dcat + H : nullptr, 2 * H)))) return rc;       // s_t
-        if ((rc = dense(n, H, H, B.h2, H, WT_(3), H, B_(3), act, B.cat, 2 * H, nullptr, 0, 1, st, nr, D_(mx, B.dcat, 2 * H)))) return rc;           // s_x
+        if ((rc = dense(n, t0, t1, B.h0, t0, WT_(1), t0, B_(1), act, B.cat + x1, C, nullptr, 0, 1, st, nr, D_(mt, dmul ? B.dcat + x1 : nullptr, C)))) return rc;       // s_t
+        if ((rc = dense(n, x0, x1, B.h2, x0, WT_(3), x0, B_(3), act, B.cat, C, nullptr, 0, 1, st, nr, D_(mx, B.dcat, C)))) return rc;           // s_x
     }
-    if ((rc = dense(n, H, d, B.cat + H, 2 * H, WT_(4), H, B_(4), 0, B.gt, d, nullptr, 0, 1, st, nr, IN_(A_(slot(AM_ST), nullptr, 0, nullptr), B.cat_s + H, BD(AM_ST))))) return rc;       // nn_t
-    if ((rc = dense(n, 2 * H, H, B.cat, 2 * H, WT_(5), 2 * H, B_(5), act, B.h5, H, nullptr, 0, 1, st, nr,
-                    D_(OUT_(IN_(A_(slot(AM_SX), slot(AM_ST), 0, slot(AM_H5)), B.cat_s, BD(AM_SX)), B.h5_s, AM_H5, 5, true), B.dh5, H)))) return rc;
-    if ((rc = dense(n, H, H, B.h5, H, WT_(6), H, B_(6), act, B.h6, H, nullptr, 0, 1, st, nr,
-                    D_(OUT_(IN_(A_(slot(AM_H5), nullptr, 0, slot(AM_H6)), B.h5_s, BD(AM_H5)), B.h6_s, AM_H6, 6, true), B.dh6, H)))) return rc;
+    if ((rc = dense(n, t1, d, B.cat + x1, C, WT_(4), t1, B_(4), 0, B.gt, d, nullptr, 0, 1, st, nr, IN_(A_(slot(AM_ST), nullptr, 0, nullptr), B.cat_s + x1, BD(AM_ST))))) return rc;       // nn_t
+    if ((rc = dense(n, C, xt0, B.cat, C, WT_(5), C, B_(5), act, B.h5, xt0, nullptr, 0, 1, st, nr,
+                    D_(OUT_(IN_(A_(slot(AM_SX), slot(AM_ST), 0, slot(AM_H5)), B.cat_s, BD(AM_SX)), B.h5_s, AM_H5, 5, true), B.dh5, xt0)))) return rc;
+    if ((rc = dense(n, xt0, xt1, B.h5, xt0, WT_(6), xt0, B_(6), act, B.h6, xt1, nullptr, 0, 1, st, nr,
+                    D_(OUT_(IN_(A_(slot(AM_H5), nullptr, 0, slot(AM_H6)), B.h5_s, BD(AM_H5)), B.h6_s, AM_H6, 6, true), B.dh6, xt1)))) return rc;
     // untempered grad logprob (clipped) and the Hessian term of the divergence
     mfm_target_t T1 = T; T1.beta = 1.0f;
     const bool want_div = out_l != nullptr;
     if ((rc = target_field_terms(T1, n, x, z, B.zkinv, F.grad_clip, B.gc, (want_div && z) ? B.hx : nullptr,
                                  (want_div && !z) ? B.hx : nullptr, nr, st, x_amax, B.tscratch, sp ? x_split : nullptr))) return rc;
     {
-        GemmShape p{n, d, H, B.h6, (long long)H, WT_(7), (long long)H, nr};
+        GemmShape p{n, d, xt1, B.h6, (long long)xt1, WT_(7), (long long)xt1, nr};
         p.a_amax = slot(AM_H6);
         if (sp) { p.a_split = B.h6_s; p.a_scale_src = BD(AM_H6); }
         EpiFieldV e{out_v, (long long)d, B_(7), B.gt, B.gc, (long long)d, sgn, row_map};
@@ -591,6 +606,7 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
         // tangent of the probe through the x branch: z W2 (per-solve constant, its exact maximum in AM_ZW2 when the caller
         // tracked it) gated by relu'(h2); gating only zeroes entries, so that maximum also scales the pre-split copy
         const bool spt = sp && zw2_amax != nullptr;
+        const int H = x0;
         if (H % 4 == 0 && ((reinterpret_cast<uintptr_t>(B.zw2) | reinterpret_cast<uintptr_t>(B.h2) | reinterpret_cast<uintptr_t>(B.ta)) & 15) == 0)
             gate4_kernel<<<ceil_div((long long)n * (H / 4), 256), 256, 0, st>>>((long long)n * (H / 4), H / 4, reinterpret_cast<const float4*>(B.zw2),
                                                                                 reinterpret_cast<const float4*>(g_h2), H / 4, reinterpret_cast<float4*>(B.ta), nr, slot(AM_TA0),
@@ -601,12 +617,12 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
         const bool vec_gate = spt && H % 4 == 0 && ((reinterpret_cast<uintptr_t>(B.zw2) | reinterpret_cast<uintptr_t>(B.h2) | reinterpret_cast<uintptr_t>(B.ta)) & 15) == 0;
         DenseAmax m1 = OUT_(A_(slot(AM_TA0), nullptr, 0, slot(AM_TB0)), B.tb_s, AM_TB0, 3, false);
         if (vec_gate) { m1.a_split = B.ta_s; m1.a_scale_src = zw2_amax; }
-        if ((rc = dense(n, H, H, B.ta, H, WT_(3), H, nullptr, 0, B.tb, H, g_cat, 2 * H, 1, st, nr, M_(m1)))) return rc;
-        if ((rc = dense(n, H, H, B.tb, H, WT_(5), 2 * H, nullptr, 0, B.ta, H, g_h5, H, 1, st, nr,
-                        M_(OUT_(IN_(A_(slot(AM_TB0), nullptr, 0, slot(AM_TA1)), B.tb_s, BD(AM_TB0)), B.ta_s, AM_TA1, 5, false))))) return rc;   // first H rows of W5
-        if ((rc = dense(n, H, H, B.ta, H, WT_(6), H, nullptr, 0, B.tb, H, g_h6, H, 1, st, nr,
+        if ((rc = dense(n, x0, x1, B.ta, x0, WT_(3), x0, nullptr, 0, B.tb, x1, g_cat, C, 1, st, nr, M_(m1)))) return rc;
+        if ((rc = dense(n, x1, xt0, B.tb, x1, WT_(5), C, nullptr, 0, B.ta, xt0, g_h5, xt0, 1, st, nr,
+                        M_(OUT_(IN_(A_(slot(AM_TB0), nullptr, 0, slot(AM_TA1)), B.tb_s, BD(AM_TB0)), B.ta_s, AM_TA1, 5, false))))) return rc;   // first x1 rows of W5
+        if ((rc = dense(n, xt0, xt1, B.ta, xt0, WT_(6), xt0, nullptr, 0, B.tb, xt1, g_h6, xt1, 1, st, nr,
                         M_(OUT_(IN_(A_(slot(AM_TA1), nullptr, 0, slot(AM_TB1)), B.ta_s, BD(AM_TA1)), B.tb_s, AM_TB1, 6, false))))) return rc;
-        GemmShape p{n, d, H, B.tb, (long long)H, WT_(7), (long long)H, nr};
+        GemmShape p{n, d, xt1, B.tb, (long long)xt1, WT_(7), (long long)xt1, nr};
         p.a_amax = slot(AM_TB1);
         if (sp) { p.a_split = B.tb_s; p.a_scale_src = BD(AM_TB1); }
         const int nt = gemm_n_tiles(d);
@@ -618,14 +634,14 @@ int field_eval(const mfm_field_t& F, const mfm_target_t& T, int n, const float* 
         const long long rows = (long long)n * d;
         if (rows > 0x7FFFFFFFll) { mfm_set_last_error_msg("exact divergence: n*d too large"); return MFM_ERR_UNSUPPORTED; }
         if (nr) { mfm_set_last_error_msg("internal: compaction is not used with the exact divergence"); return MFM_ERR_UNSUPPORTED; }
-        basis_tangent_kernel<<<ceil_div(rows * H, 256), 256, 0, st>>>(n, d, H, W_(2), g_h2, B.tan_a, nullptr, dmul ? 1 : 0);
+        basis_tangent_kernel<<<ceil_div(rows * x0, 256), 256, 0, st>>>(n, d, x0, W_(2), g_h2, B.tan_a, nullptr, dmul ? 1 : 0);
         MFM_LAUNCH_CHECK();
         // the basis tangents are entries of W2 or zero (relu): max |parameter| bounds them; the other activations' derivatives
         // reach 1.13 (gelu), so their tangents get an on-the-fly maximum instead
-        if ((rc = dense((int)rows, H, H, B.tan_a, H, WT_(3), H, nullptr, 0, B.tan_b, H, g_cat, 2 * H, d, st, nullptr, M_(A_(dmul ? nullptr : slot(AM_W), nullptr, 0, slot(AM_TB0)))))) return rc;
-        if ((rc = dense((int)rows, H, H, B.tan_b, H, WT_(5), 2 * H, nullptr, 0, B.tan_a, H, g_h5, H, d, st, nullptr, M_(A_(slot(AM_TB0), nullptr, 0, slot(AM_TA1)))))) return rc;
-        if ((rc = dense((int)rows, H, H, B.tan_a, H, WT_(6), H, nullptr, 0, B.tan_b, H, g_h6, H, d, st, nullptr, M_(A_(slot(AM_TA1), nullptr, 0, nullptr))))) return rc;
-        exact_trace_kernel<<<ceil_div(n, 8), 256, 0, st>>>(n, d, H, B.tan_b, W_(7), B.gt, B.hx, -sgn, out_l, nullptr, row_map);
+        if ((rc = dense((int)rows, x0, x1, B.tan_a, x0, WT_(3), x0, nullptr, 0, B.tan_b, x1, g_cat, C, d, st, nullptr, M_(A_(dmul ? nullptr : slot(AM_W), nullptr, 0, slot(AM_TB0)))))) return rc;
+        if ((rc = dense((int)rows, x1, xt0, B.tan_b, x1, WT_(5), C, nullptr, 0, B.tan_a, xt0, g_h5, xt0, d, st, nullptr, M_(A_(slot(AM_TB0), nullptr, 0, slot(AM_TA1)))))) return rc;
+        if ((rc = dense((int)rows, xt0, xt1, B.tan_a, xt0, WT_(6), xt0, nullptr, 0, B.tan_b, xt1, g_h6, xt1, d, st, nullptr, M_(A_(slot(AM_TA1), nullptr, 0, nullptr))))) return rc;
+        exact_trace_kernel<<<ceil_div(n, 8), 256, 0, st>>>(n, d, xt1, B.tan_b, W_(7), B.gt, B.hx, -sgn, out_l, nullptr, row_map);
         MFM_LAUNCH_CHECK();
     }
     return MFM_OK;
@@ -1054,7 +1070,7 @@ static int* host_flag() {
 static int ode_solve(const mfm_field_t& F, const mfm_target_t& T, const mfm_ode_opts_t& O, int direction, int n,
                      const float* z, const float* y0, float* y1, float* ldj, int* stats, int stats_accumulate,
                      OdeState& S, FieldBufs& B, float* z_compact, cudaStream_t st, float z_bound = NORMAL_BOUND) {
-    const int d = F.dim, H = F.hidden;
+    const int d = F.dim, H = field_widths(F).x0;         // width of the probe constant z W2
     const float sgn = direction >= 0 ? 1.0f : -1.0f;
     if (O.n_times < 2 || O.n_times > 17) { mfm_set_last_error_msg("n_times must be in [2,17]"); return MFM_ERR_ARG; }
     OdeTimes TS; TS.n_seg = O.n_times - 1;
@@ -1390,13 +1406,14 @@ static int check_field(const mfm_field_t* f, const mfm_target_t* t, const mfm_od
     if (f->dim != t->dim) { mfm_set_last_error_msg("field.dim != target.dim"); return MFM_ERR_ARG; }
     if (f->hidden <= 0 || f->fourier_dim <= 0 || !f->params || !f->omega) { mfm_set_last_error_msg("bad field descriptor"); return MFM_ERR_ARG; }
     if (f->act < MFM_ACT_RELU || f->act > MFM_ACT_SWISH) { mfm_set_last_error_msg("unknown activation (mfm_field_t::act)"); return MFM_ERR_ARG; }
+    if (int rc = field_widths_check(f)) return rc;
     return ref_check(f, false);
 }
 
 void mfm_debug_set_ode_small(int v) { g_ode_small = v ? 1 : 0; }      // test hook (not in the ABI header): fused small-shape solve on / off
 
 size_t mfm_ode_workspace_bytes(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_opts_t* o, int n) {
-    return ode_state_bytes(n, f->dim, f->hidden) + field_bufs_bytes(*f, *t, n, o->hutch != 0) + 2 * ws_slice((size_t)n * f->dim, 4) + 1024;
+    return ode_state_bytes(n, f->dim, field_widths(*f).x0) + field_bufs_bytes(*f, *t, n, o->hutch != 0) + 2 * ws_slice((size_t)n * f->dim, 4) + 1024;
 }
 
 int mfm_ode_flow(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_opts_t* o, int direction, int n,
@@ -1408,7 +1425,7 @@ int mfm_ode_flow(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_opts
     if (n <= 0) return MFM_OK;
     Workspace w(ws, ws_bytes);
     OdeState S; FieldBufs B;
-    ode_state_take(S, w, n, f->dim, f->hidden);
+    ode_state_take(S, w, n, f->dim, field_widths(*f).x0);
     field_bufs_take(B, w, *f, n, o->hutch != 0, t);
     float* z = nullptr; float* zc = nullptr;
     if (o->hutch) { z = w.take<float>((size_t)n * f->dim); zc = w.take<float>((size_t)n * f->dim); }
@@ -1467,7 +1484,7 @@ int mfm_flow_mh_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode_
     const size_t N = n, D = d;
     Workspace w(ws, ws_bytes);
     OdeState S; FieldBufs B;
-    ode_state_take(S, w, n, d, f->hidden);
+    ode_state_take(S, w, n, d, field_widths(*f).x0);
     field_bufs_take(B, w, *f, n, o->hutch != 0, t);
     float* z = w.take<float>(N * D); float* zc = w.take<float>(N * D);
     float* u0 = w.take<float>(N * D); float* up = w.take<float>(N * D); float* xp = w.take<float>(N * D);
@@ -1537,7 +1554,7 @@ int mfm_flow_cis_step(const mfm_field_t* f, const mfm_target_t* t, const mfm_ode
     const bool hutch = o->hutch != 0;
     Workspace w(ws, ws_bytes);
     OdeState S; FieldBufs B;
-    ode_state_take(S, w, M, d, f->hidden);
+    ode_state_take(S, w, M, d, field_widths(*f).x0);
     field_bufs_take(B, w, *f, M, hutch, t);
     float* z = w.take<float>(MM * D); float* zc = w.take<float>(MM * D);
     float* refs = w.take<float>(MM * D); float* samples = w.take<float>(MM * D); float* gscr = w.take<float>(MM * D);

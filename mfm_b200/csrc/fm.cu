@@ -383,34 +383,41 @@ struct FmBufs {
 static const int FM_LOSS_BLOCKS = 1024;
 
 static size_t fm_splitbuf_floats(const mfm_field_t& F) {
-    const size_t H = F.hidden, d = F.dim, Fd = F.fourier_dim;
-    size_t m = 2 * H * H;
-    if (d * H > m) m = d * H;
-    if (2 * Fd * H > m) m = 2 * Fd * H;
+    const FieldWidths W = field_widths(F);
+    const size_t d = F.dim, Fd = F.fourier_dim;
+    const size_t layer[8] = {2 * Fd * W.t0, (size_t)W.t0 * W.t1, d * W.x0, (size_t)W.x0 * W.x1, (size_t)W.t1 * d, (size_t)W.cat() * W.xt0,
+                             (size_t)W.xt0 * W.xt1, (size_t)W.xt1 * d};
+    size_t m = 0;
+    for (int i = 0; i < 8; ++i) m = layer[i] > m ? layer[i] : m;
     return m * 16;     // room for 16 batch slices of the largest layer (more for smaller ones)
 }
 
+// the back-propagated signals: d6 [n, xt1], d5 [n, xt0], d2 [n, x0], d0 [n, t0], dcat [n, x1 + t1] (and as many pre-split copies);
+// the column-sum partials hold the widest of them
 static size_t fm_bytes(const mfm_field_t& F, const mfm_target_t& T, int n) {
-    const size_t H = F.hidden, d = F.dim, N = n;
-    return field_bufs_bytes(F, T, n, true) + ws_slice(N, 4) + ws_slice(N * d, 4) * 5 + ws_slice(N * H, 4) * 4 +
-           ws_slice(N * 2 * H, 4) + ws_slice(FM_LOSS_BLOCKS, 4) + ws_slice(fm_splitbuf_floats(F), 4) +
-           ws_slice((size_t)COLSUM_SLABS * (H > d ? H : d), 4) + ws_slice(N * H, 4) * 4 + ws_slice(N * 2 * H, 4) + ws_slice(N * d, 4) * 3 + ws_slice(((N + 31) / 32) * H, 4) + 1024;
+    const FieldWidths W = field_widths(F);
+    const size_t H = W.widest(), d = F.dim, N = n;
+    const size_t sig = ws_slice(N * W.xt1, 4) + ws_slice(N * W.xt0, 4) + ws_slice(N * W.x0, 4) + ws_slice(N * W.t0, 4) + ws_slice(N * W.cat(), 4);
+    return field_bufs_bytes(F, T, n, true) + ws_slice(N, 4) + ws_slice(N * d, 4) * 5 + sig + ws_slice(FM_LOSS_BLOCKS, 4) +
+           ws_slice(fm_splitbuf_floats(F), 4) + ws_slice((size_t)COLSUM_SLABS * (H > d ? H : d), 4) + sig + ws_slice(N * d, 4) * 3 +
+           ws_slice(((N + 31) / 32) * H, 4) + 1024;
 }
 
 static bool fm_take(FmBufs& M, Workspace& w, const mfm_field_t& F, int n, const mfm_target_t* T) {
-    const size_t H = F.hidden, d = F.dim, N = n;
+    const FieldWidths W = field_widths(F);
+    const size_t H = W.widest(), d = F.dim, N = n, C = W.cat();
     field_bufs_take(M.B, w, F, n, true, T);
     M.times = w.take<float>(N);
     M.xt = w.take<float>(N * d); M.target = w.take<float>(N * d); M.v = w.take<float>(N * d);
     M.delta = w.take<float>(N * d); M.dgt = w.take<float>(N * d);
-    M.d6 = w.take<float>(N * H); M.d5 = w.take<float>(N * H); M.d2 = w.take<float>(N * H); M.d0 = w.take<float>(N * H);
-    M.dcat = w.take<float>(N * 2 * H);
+    M.d6 = w.take<float>(N * W.xt1); M.d5 = w.take<float>(N * W.xt0); M.d2 = w.take<float>(N * W.x0); M.d0 = w.take<float>(N * W.t0);
+    M.dcat = w.take<float>(N * C);
     M.blockpart = w.take<float>(FM_LOSS_BLOCKS);
     M.colpart = w.take<float>((size_t)COLSUM_SLABS * (H > d ? H : d));
     M.splitbuf_floats = fm_splitbuf_floats(F);
     M.splitbuf = w.take<float>(M.splitbuf_floats);
-    M.d6_s = w.take<float>(N * H); M.d5_s = w.take<float>(N * H); M.dcat_s = w.take<float>(N * 2 * H);
-    M.d2_s = w.take<float>(N * H); M.d0_s = w.take<float>(N * H);
+    M.d6_s = w.take<float>(N * W.xt1); M.d5_s = w.take<float>(N * W.xt0); M.dcat_s = w.take<float>(N * C);
+    M.d2_s = w.take<float>(N * W.x0); M.d0_s = w.take<float>(N * W.t0);
     M.xt_s = w.take<float>(N * d); M.delta_s = w.take<float>(N * d); M.dgt_s = w.take<float>(N * d);
     M.cspart = w.take<float>(((N + 31) / 32) * H);
     return w.ok;
@@ -446,7 +453,9 @@ static FmAux* fm_aux() {
 // xt_amax: slot holding max |x_t| when the batch kernel tracked it (null: field_eval reduces it).
 static int fm_forward_backward(const mfm_field_t& F, const mfm_target_t& T, int n, FmBufs& M, float* loss_out,
                                float* grads, cudaStream_t st, int part, const float* xt_amax = nullptr, bool tgt_tracked = false) {
-    const int d = F.dim, H = F.hidden, Fd = F.fourier_dim;
+    const int d = F.dim, Fd = F.fourier_dim;
+    const FieldWidths W = field_widths(F);
+    const int t0 = W.t0, t1 = W.t1, x0 = W.x0, x1 = W.x1, xt0 = W.xt0, xt1 = W.xt1, C = W.cat();   // cat / dcat: [n, x1 + t1], s_t from column x1
     FieldBufs& B = M.B;
     int rc;
     if (part == 2) field_register_mirrors(F, B);      // built by part 1 in this workspace
@@ -456,7 +465,7 @@ static int fm_forward_backward(const mfm_field_t& F, const mfm_target_t& T, int 
     // weight gradients from the split16 copies (gemm_tcgen05_wgrad16.cuh): same conditions as the copies' producers
     static const bool no_wsplit = getenv("MFM_H16_NOWGRAD") != nullptr;
     static const bool no_split = getenv("MFM_H16_NOSPLIT") != nullptr;
-    const bool wsp = !no_wsplit && !no_split && am != nullptr && M.d6_s != nullptr && B.h0_s != nullptr && H % 16 == 0 && (2 * Fd) % 16 == 0 && n >= 256 &&
+    const bool wsp = !no_wsplit && !no_split && am != nullptr && M.d6_s != nullptr && B.h0_s != nullptr && W.all16() && (2 * Fd) % 16 == 0 && n >= 256 &&
                      ((reinterpret_cast<uintptr_t>(B.h0_s) | reinterpret_cast<uintptr_t>(B.cat_s)) & 63) == 0;
     const bool wspd = wsp && d % 16 == 0;      // the [n, d] operands have copies too
     // the loss kernel writes delta / dgt pre-split itself when it can bound them beforehand (tracked maxima of v and of the
@@ -531,7 +540,7 @@ static int fm_forward_backward(const mfm_field_t& F, const mfm_target_t& T, int 
     bool cs6 = false, cs5 = false, csx = false, cst = false, cs2 = false, cs0 = false;
     float* sb = M.splitbuf; const size_t sbf = M.splitbuf_floats;
     // pre-split copies along the backward-data chain (as in field_eval): slot ids of the exact maxima / bounds, ROW norms of the kernels
-    const bool sp = am != nullptr && M.d6_s != nullptr && H % 16 == 0 && n >= 256;
+    const bool sp = am != nullptr && M.d6_s != nullptr && W.all16() && n >= 256;
     auto BD = [&](int i) -> float* { return am + AM_BOUND + i; };
     auto WR = [&](int l) -> const float* { return am + AM_WNORM_ROW + l; };
     // (exact max of D, [D pre-split, slot of its scale]) -> exact max of dX [, dX pre-split, slot of its bound, layer, bound of `add`]
@@ -574,50 +583,50 @@ static int fm_forward_backward(const mfm_field_t& F, const mfm_target_t& T, int 
     if (part != 2) {
     // layer 7 (nn_xt head): y = h6 W7 + b7
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, H, d, B.h6, H, M.delta, d, GW_(7), sb, sbf, sw, WS_(wspd, B.h6_s, BD(AM_H6), M.delta_s, delta_src)))) return rc;
+    if ((rc = wgrad(n, xt1, d, B.h6, xt1, M.delta, d, GW_(7), sb, sbf, sw, WS_(wspd, B.h6_s, BD(AM_H6), M.delta_s, delta_src)))) return rc;
     if ((rc = bias_grad(M.delta, d, d, GB_(7)))) return rc;
-    if ((rc = dgrad(n, H, d, M.delta, d, W_(7), M.d6, H, g_h6, H, nullptr, 0, st, G_(slot(AM_DELTA), fused_loss ? M.delta_s : nullptr, delta_src, slot(AM_D6), M.d6_s, AM_D6, 7, nullptr), M.cspart, &cs6))) return rc;
-    if ((rc = bias_grad_cs(cs6, M.d6, H, H, GB_(6)))) return rc;        // bias gradients: column sums of the signal just written
+    if ((rc = dgrad(n, xt1, d, M.delta, d, W_(7), M.d6, xt1, g_h6, xt1, nullptr, 0, st, G_(slot(AM_DELTA), fused_loss ? M.delta_s : nullptr, delta_src, slot(AM_D6), M.d6_s, AM_D6, 7, nullptr), M.cspart, &cs6))) return rc;
+    if ((rc = bias_grad_cs(cs6, M.d6, xt1, xt1, GB_(6)))) return rc;        // bias gradients: column sums of the signal just written
     // layer 6
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, H, H, B.h5, H, M.d6, H, GW_(6), sb, sbf, sw, WS_(wsp, B.h5_s, BD(AM_H5), M.d6_s, BD(AM_D6))))) return rc;
-    if ((rc = dgrad(n, H, H, M.d6, H, W_(6), M.d5, H, g_h5, H, nullptr, 0, st, G_(slot(AM_D6), M.d6_s, BD(AM_D6), slot(AM_D5), M.d5_s, AM_D5, 6, nullptr), M.cspart, &cs5))) return rc;
-    if ((rc = bias_grad_cs(cs5, M.d5, H, H, GB_(5)))) return rc;
+    if ((rc = wgrad(n, xt0, xt1, B.h5, xt0, M.d6, xt1, GW_(6), sb, sbf, sw, WS_(wsp, B.h5_s, BD(AM_H5), M.d6_s, BD(AM_D6))))) return rc;
+    if ((rc = dgrad(n, xt0, xt1, M.d6, xt1, W_(6), M.d5, xt0, g_h5, xt0, nullptr, 0, st, G_(slot(AM_D6), M.d6_s, BD(AM_D6), slot(AM_D5), M.d5_s, AM_D5, 6, nullptr), M.cspart, &cs5))) return rc;
+    if ((rc = bias_grad_cs(cs5, M.d5, xt0, xt0, GB_(5)))) return rc;
     // layer 5 (joint, input cat = [s_x | s_t])
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, 2 * H, H, B.cat, 2 * H, M.d5, H, GW_(5), sb, sbf, sw, WS_(wsp, B.cat_s, BD(AM_SX), M.d5_s, BD(AM_D5))))) return rc;
-    // d s_x = (d5 W5[:H]^T) * relu'(s_x)
-    if ((rc = dgrad(n, H, H, M.d5, H, W_(5), M.dcat, 2 * H, g_cat, 2 * H, nullptr, 0, st, G_(slot(AM_D5), M.d5_s, BD(AM_D5), slot(AM_DCX), M.dcat_s, AM_DCX, 5, nullptr), M.cspart, &csx))) return rc;
-    if ((rc = bias_grad_cs(csx, M.dcat, 2 * H, H, GB_(3)))) return rc;  // (layer 3's bias; its slot lies in the head of the flat buffer, which nobody reads before part 2 ends)
-    // d s_t (joint part) = d5 W5[H:]^T   (no gate yet; its bound enters the next layer's through `add`)
-    if ((rc = dgrad(n, H, H, M.d5, H, W_(5) + (long long)H * H, M.dcat + H, 2 * H, nullptr, 0, nullptr, 0, st,
-                    G_(slot(AM_D5), M.d5_s, BD(AM_D5), nullptr, M.dcat_s + H, AM_DCT0, 5, nullptr)))) return rc;
+    if ((rc = wgrad(n, C, xt0, B.cat, C, M.d5, xt0, GW_(5), sb, sbf, sw, WS_(wsp, B.cat_s, BD(AM_SX), M.d5_s, BD(AM_D5))))) return rc;
+    // d s_x = (d5 W5[:x1]^T) * relu'(s_x)
+    if ((rc = dgrad(n, x1, xt0, M.d5, xt0, W_(5), M.dcat, C, g_cat, C, nullptr, 0, st, G_(slot(AM_D5), M.d5_s, BD(AM_D5), slot(AM_DCX), M.dcat_s, AM_DCX, 5, nullptr), M.cspart, &csx))) return rc;
+    if ((rc = bias_grad_cs(csx, M.dcat, C, x1, GB_(3)))) return rc;  // (layer 3's bias; its slot lies in the head of the flat buffer, which nobody reads before part 2 ends)
+    // d s_t (joint part) = d5 W5[x1:]^T   (no gate yet; its bound enters the next layer's through `add`)
+    if ((rc = dgrad(n, t1, xt0, M.d5, xt0, W_(5) + (long long)x1 * xt0, M.dcat + x1, C, nullptr, 0, nullptr, 0, st,
+                    G_(slot(AM_D5), M.d5_s, BD(AM_D5), nullptr, M.dcat_s + x1, AM_DCT0, 5, nullptr)))) return rc;
     // layer 4 (nn_t head): g_t = s_t W4 + b4, dL/dg_t = delta * clip(grad logprob)
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, H, d, B.cat + H, 2 * H, M.dgt, d, GW_(4), sb, sbf, sw, WS_(wspd, B.cat_s + H, BD(AM_ST), M.dgt_s, dgt_src)))) return rc;
+    if ((rc = wgrad(n, t1, d, B.cat + x1, C, M.dgt, d, GW_(4), sb, sbf, sw, WS_(wspd, B.cat_s + x1, BD(AM_ST), M.dgt_s, dgt_src)))) return rc;
     if ((rc = bias_grad(M.dgt, d, d, GB_(4)))) return rc;
     // d s_t = (dgt W4^T + joint part) * relu'(s_t)   (in place)
-    if ((rc = dgrad(n, H, d, M.dgt, d, W_(4), M.dcat + H, 2 * H, g_cat + H, 2 * H, M.dcat + H, 2 * H, st,
-                    G_(slot(AM_DGT), fused_loss ? M.dgt_s : nullptr, dgt_src, slot(AM_DCT), M.dcat_s + H, AM_DCT, 4, sp ? BD(AM_DCT0) : nullptr), M.cspart, &cst))) return rc;
-    if ((rc = bias_grad_cs(cst, M.dcat + H, 2 * H, H, GB_(1)))) return rc;
+    if ((rc = dgrad(n, t1, d, M.dgt, d, W_(4), M.dcat + x1, C, g_cat + x1, C, M.dcat + x1, C, st,
+                    G_(slot(AM_DGT), fused_loss ? M.dgt_s : nullptr, dgt_src, slot(AM_DCT), M.dcat_s + x1, AM_DCT, 4, sp ? BD(AM_DCT0) : nullptr), M.cspart, &cst))) return rc;
+    if ((rc = bias_grad_cs(cst, M.dcat + x1, C, t1, GB_(1)))) return rc;
     }
     if (part == 1) return join_w();
     // layer 3 (x branch)
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, H, H, B.h2, H, M.dcat, 2 * H, GW_(3), sb, sbf, sw, WS_(wsp && xa_src, B.h2_s, BD(AM_H2), M.dcat_s, BD(AM_DCX))))) return rc;
-    if ((rc = dgrad(n, H, H, M.dcat, 2 * H, W_(3), M.d2, H, g_h2, H, nullptr, 0, st, G_(slot(AM_DCX), M.dcat_s, BD(AM_DCX), slot(AM_D2), wsp ? M.d2_s : nullptr, AM_D2, 3, nullptr), M.cspart, &cs2))) return rc;
-    if ((rc = bias_grad_cs(cs2, M.d2, H, H, GB_(2)))) return rc;
+    if ((rc = wgrad(n, x0, x1, B.h2, x0, M.dcat, C, GW_(3), sb, sbf, sw, WS_(wsp && xa_src, B.h2_s, BD(AM_H2), M.dcat_s, BD(AM_DCX))))) return rc;
+    if ((rc = dgrad(n, x0, x1, M.dcat, C, W_(3), M.d2, x0, g_h2, x0, nullptr, 0, st, G_(slot(AM_DCX), M.dcat_s, BD(AM_DCX), slot(AM_D2), wsp ? M.d2_s : nullptr, AM_D2, 3, nullptr), M.cspart, &cs2))) return rc;
+    if ((rc = bias_grad_cs(cs2, M.d2, x0, x0, GB_(2)))) return rc;
     // layer 2
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, d, H, M.xt, d, M.d2, H, GW_(2), sb, sbf, sw, WS_(wspd && xa_src, M.xt_s, xa_src, M.d2_s, BD(AM_D2))))) return rc;
+    if ((rc = wgrad(n, d, x0, M.xt, d, M.d2, x0, GW_(2), sb, sbf, sw, WS_(wspd && xa_src, M.xt_s, xa_src, M.d2_s, BD(AM_D2))))) return rc;
     // layer 1 (time branch)
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, H, H, B.h0, H, M.dcat + H, 2 * H, GW_(1), sb, sbf, sw, WS_(wsp, B.h0_s, BD(AM_H0), M.dcat_s + H, BD(AM_DCT))))) return rc;
-    if ((rc = dgrad(n, H, H, M.dcat + H, 2 * H, W_(1), M.d0, H, g_h0, H, nullptr, 0, st, G_(slot(AM_DCT), M.dcat_s + H, BD(AM_DCT), slot(AM_D0), wsp ? M.d0_s : nullptr, AM_D0, 1, nullptr), M.cspart, &cs0))) return rc;
-    if ((rc = bias_grad_cs(cs0, M.d0, H, H, GB_(0)))) return rc;
+    if ((rc = wgrad(n, t0, t1, B.h0, t0, M.dcat + x1, C, GW_(1), sb, sbf, sw, WS_(wsp, B.h0_s, BD(AM_H0), M.dcat_s + x1, BD(AM_DCT))))) return rc;
+    if ((rc = dgrad(n, t0, t1, M.dcat + x1, C, W_(1), M.d0, t0, g_h0, t0, nullptr, 0, st, G_(slot(AM_DCT), M.dcat_s + x1, BD(AM_DCT), slot(AM_D0), wsp ? M.d0_s : nullptr, AM_D0, 1, nullptr), M.cspart, &cs0))) return rc;
+    if ((rc = bias_grad_cs(cs0, M.d0, t0, t0, GB_(0)))) return rc;
     // layer 0
     if ((rc = fork_w())) return rc;
-    if ((rc = wgrad(n, 2 * Fd, H, B.ff, 2 * Fd, M.d0, H, GW_(0), sb, sbf, sw, WS_(wsp, B.ff_s, BD(AM_FF), M.d0_s, BD(AM_D0))))) return rc;
+    if ((rc = wgrad(n, 2 * Fd, t0, B.ff, 2 * Fd, M.d0, t0, GW_(0), sb, sbf, sw, WS_(wsp, B.ff_s, BD(AM_FF), M.d0_s, BD(AM_D0))))) return rc;
     return join_w();
 }
 
@@ -693,6 +702,7 @@ size_t mfm_fm_workspace_bytes(const mfm_field_t* f, const mfm_target_t* t, int n
 static int fm_check(const mfm_field_t* f, const mfm_target_t* t, bool samples_ref = false) {
     if (!f || !t) { mfm_set_last_error_msg("null descriptor"); return MFM_ERR_ARG; }
     if (f->dim != t->dim) { mfm_set_last_error_msg("field.dim != target.dim"); return MFM_ERR_ARG; }
+    if (int rc = field_widths_check(f)) return rc;
     return ref_check(f, samples_ref);
 }
 

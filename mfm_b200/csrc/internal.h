@@ -43,6 +43,40 @@ int target_field_terms(const mfm_target_t& T, int n, const float* x, const float
                        float* scratch = nullptr, const float* x_split = nullptr);
 
 // ---- vector field (flow.cu) -------------------------------------------------------------------
+// Hidden widths of the eight dense layers (mfm_field_t::hidden_t / hidden_x / hidden_xt; an all-zero tail: every width is
+// `hidden`).  Dense_0 2F->t0, Dense_1 t0->t1, Dense_2 d->x0, Dense_3 x0->x1, Dense_4 t1->d, Dense_5 (x1 + t1)->xt0 over
+// cat = [s_x | s_t], Dense_6 xt0->xt1, Dense_7 xt1->d.  Negative entries of a malformed tail are read as 0 here (buffer sizes
+// only): field_widths_check refuses the descriptor before anything runs.
+struct FieldWidths {
+    int t0, t1, x0, x1, xt0, xt1;
+    bool equal;                                                   // all six == hidden (today's network)
+    int cat() const { return x1 + t1; }                           // row stride of cat / dcat; s_t starts at column x1
+    int tan() const { int m = x0 > x1 ? x0 : x1; m = m > xt0 ? m : xt0; return m > xt1 ? m : xt1; }   // tangents: x and joint branches
+    int widest() const { const int m = tan(); return m > t0 ? (m > t1 ? m : t1) : (t0 > t1 ? t0 : t1); }
+    int narrowest() const { int m = t0 < t1 ? t0 : t1; m = m < x0 ? m : x0; m = m < x1 ? m : x1; m = m < xt0 ? m : xt0; return m < xt1 ? m : xt1; }
+    bool all16() const { return t0 % 16 == 0 && t1 % 16 == 0 && x0 % 16 == 0 && x1 % 16 == 0 && xt0 % 16 == 0 && xt1 % 16 == 0; }
+};
+inline FieldWidths field_widths(const mfm_field_t& F) {
+    FieldWidths w;
+    const int* v[3] = {F.hidden_t, F.hidden_x, F.hidden_xt};
+    bool zero = true;
+    for (int b = 0; b < 3; ++b) zero = zero && v[b][0] == 0 && v[b][1] == 0;
+    auto g = [&](int b, int i) { return zero ? F.hidden : (v[b][i] > 0 ? v[b][i] : 0); };
+    w.t0 = g(0, 0); w.t1 = g(0, 1); w.x0 = g(1, 0); w.x1 = g(1, 1); w.xt0 = g(2, 0); w.xt1 = g(2, 1);
+    w.equal = w.t0 == F.hidden && w.t1 == F.hidden && w.x0 == F.hidden && w.x1 == F.hidden && w.xt0 == F.hidden && w.xt1 == F.hidden;
+    return w;
+}
+// MFM_ERR_ARG (with a message) unless the width tail is all zero, or all positive with `hidden` the largest
+inline int field_widths_check(const mfm_field_t* f) {
+    const int* v[3] = {f->hidden_t, f->hidden_x, f->hidden_xt};
+    int n_zero = 0, n_pos = 0, widest = 0;
+    for (int b = 0; b < 3; ++b)
+        for (int i = 0; i < 2; ++i) { n_zero += v[b][i] == 0; n_pos += v[b][i] > 0; widest = v[b][i] > widest ? v[b][i] : widest; }
+    if (n_zero == 6) return 0;
+    if (n_pos != 6) { mfm_set_last_error_msg("field.hidden_t / hidden_x / hidden_xt: all six widths must be > 0 (or all 0: every width is `hidden`)"); return MFM_ERR_ARG; }
+    if (f->hidden != widest) { mfm_set_last_error_msg("field.hidden must equal the widest of hidden_t / hidden_x / hidden_xt"); return MFM_ERR_ARG; }
+    return 0;
+}
 // Slots of the per-workspace pool of tensor maxima (FieldBufs::amax, 64 floats): max |value| of every tensor that is the A
 // operand of a scaled-fp16 GEMM (gemm_tcgen05_h16.cuh), written by its producer with atomicMax.  Slots below AM_EVAL_END
 // are zeroed at the start of every field evaluation; the others belong to the caller of field_eval (one ODE solve / one FM

@@ -12,7 +12,7 @@
 // every 32 k (the arithmetic of gemm_tf32x3.cuh); the 16 warps split a layer's output columns, one n-tile of 8 each; the A
 // operand is split into tf32 hi / lo planes once per layer.
 // Forward-mode tangents (one Hutchinson probe, or the d basis tangents of the exact trace) reuse the same row tile, one
-// pass per tangent.  Eligibility: H in {64, 128}, d <= 16, 2F <= 256, relu / tanh / elu (their derivatives follow from the
+// pass per tangent.  Eligibility: all six hidden widths equal, H in {64, 128}, d <= 16, 2F <= 256, relu / tanh / elu (their derivatives follow from the
 // stored outputs), the warp-per-chain targets (mixture, phi-four, Gaussian).
 //
 // Before: ~120 launches per Runge-Kutta iteration (1.4 ms each at 128 chains even from a CUDA-graph loop); now the whole
@@ -458,7 +458,8 @@ __global__ void __launch_bounds__(NTHR, 1) ode_small_kernel(const Args A) {
 inline bool eligible(const mfm_field_t& F, const mfm_target_t& T, int n) {
     const bool target_ok = T.kind == MFM_TARGET_GMM || T.kind == MFM_TARGET_PHI4 || T.kind == MFM_TARGET_GAUSS;
     const bool act_ok = F.act == MFM_ACT_RELU || F.act == MFM_ACT_TANH || F.act == MFM_ACT_ELU;
-    return target_ok && act_ok && n > 0 && F.dim <= DP && (F.hidden == 64 || F.hidden == 128) && (F.fourier_dim == 32 || F.fourier_dim == 64 || F.fourier_dim == 128) && !(T.kind == MFM_TARGET_GMM && F.dim != 2);
+    // (one width for every layer: networks with unequal branch widths take the graph-driven loop of ode_solve)
+    return target_ok && act_ok && field_widths(F).equal && n > 0 && F.dim <= DP && (F.hidden == 64 || F.hidden == 128) && (F.fourier_dim == 32 || F.fourier_dim == 64 || F.fourier_dim == 128) && !(T.kind == MFM_TARGET_GMM && F.dim != 2);
 }
 
 }  // namespace small

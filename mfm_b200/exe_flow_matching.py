@@ -54,19 +54,42 @@ def make_ref_dist(args, dim, device=None):
 # ------------------------------------------------------------------------------------------------
 # VectorFieldNet
 # ------------------------------------------------------------------------------------------------
-def layer_shapes(dim: int, hidden: int, fourier_dim: int):
-    """(in, out) of Dense_0..Dense_7 in flax construction order (exe_flow_matching.py:73-86)."""
-    F, H, d = fourier_dim, hidden, dim
-    return [(2 * F, H), (H, H), (d, H), (H, H), (H, d), (2 * H, H), (H, H), (H, d)]
+def branch_widths(hidden_t, hidden_x, hidden_xt):
+    """((Ht0, Ht1), (Hx0, Hx1), (Hxt0, Hxt1)) from the three --hidden_* lists.  The device network has exactly two hidden
+    layers per branch (flax names Dense_0..Dense_7); each width is free."""
+    out = []
+    for name, ws in (("hidden_t", hidden_t), ("hidden_x", hidden_x), ("hidden_xt", hidden_xt)):
+        ws = [int(w) for w in ws]
+        if len(ws) != 2:
+            raise NotImplementedError(f"{name} has {len(ws)} layers: the CUDA path implements two hidden layers per branch "
+                                      "(depth is the limit; the widths are free)")
+        if min(ws) <= 0:
+            raise ValueError(f"{name} widths must be positive, got {ws}")
+        out.append(tuple(ws))
+    return tuple(out)
+
+
+def layer_shapes(dim: int, hidden: int, fourier_dim: int, widths=None):
+    """(in, out) of Dense_0..Dense_7 in flax construction order (exe_flow_matching.py:73-86).  widths: ((Ht0, Ht1), (Hx0, Hx1),
+    (Hxt0, Hxt1)) as branch_widths returns it; None: every width is `hidden`.  Dense_5 reads cat = [s_x | s_t]."""
+    F, d = fourier_dim, dim
+    (t0, t1), (x0, x1), (xt0, xt1) = widths if widths is not None else ((hidden,) * 2,) * 3
+    return [(2 * F, t0), (t0, t1), (d, x0), (x0, x1), (t1, d), (x1 + t1, xt0), (xt0, xt1), (xt1, d)]
 
 
 class VectorFieldParams:
     """Flat fp32 parameter buffer + offsets; converts from/to the flax dict layout
-    {'params': {'Dense_i': {'kernel': [in,out], 'bias': [out]}}}."""
+    {'params': {'Dense_i': {'kernel': [in,out], 'bias': [out]}}}.  widths (optional): the per-branch hidden widths
+    ((Ht0, Ht1), (Hx0, Hx1), (Hxt0, Hxt1)); `hidden` must then be the widest of them."""
 
-    def __init__(self, dim, hidden, fourier_dim, device):
+    def __init__(self, dim, hidden, fourier_dim, device, widths=None):
+        if widths is not None:
+            widths = branch_widths(*widths)
+            if hidden != max(max(w) for w in widths):
+                raise ValueError(f"hidden={hidden} must be the widest layer of {widths}")
         self.dim, self.hidden, self.fourier_dim = dim, hidden, fourier_dim
-        self.shapes = layer_shapes(dim, hidden, fourier_dim)
+        self.widths = widths if widths is not None else ((hidden, hidden),) * 3
+        self.shapes = layer_shapes(dim, hidden, fourier_dim, widths)
         self.w_off, self.b_off = [], []
         off = 0
         for fi, fo in self.shapes:
@@ -115,16 +138,14 @@ class VectorFieldNet:
 
     def __init__(self, fourier_random: torch.Tensor, dist: Distribution, hidden_x, hidden_t, hidden_xt,
                  act_fn="relu", grad_clip: Optional[float] = None):
-        hs = list(hidden_x) + list(hidden_t) + list(hidden_xt)
-        if len(hidden_x) != 2 or len(hidden_t) != 2 or len(hidden_xt) != 2 or len(set(hs)) != 1:
-            raise NotImplementedError("the CUDA path implements the configured shape: three 2-layer branches of equal width")
+        self.widths = branch_widths(hidden_t, hidden_x, hidden_xt)     # ((Ht0, Ht1), (Hx0, Hx1), (Hxt0, Hxt1))
         if act_fn is torch.relu:
             act_fn = "relu"
         if act_fn not in _lib.ACTIVATIONS:                       # non_lins (:40-46)
             raise KeyError(f"unknown non_linearity {act_fn!r}: one of {sorted(_lib.ACTIVATIONS)}")
         self.act = _lib.ACTIVATIONS[act_fn]
         self.dist = dist
-        self.hidden = hs[0]
+        self.hidden = max(max(w) for w in self.widths)
         self.fourier_random = fourier_random.to(torch.float32).contiguous()
         self.grad_clip = float(grad_clip) if grad_clip else 0.0
         self.ref_mean, self.ref_std = 0.0, 1.0     # reference distribution of the flow (set_ref_dist)
@@ -148,7 +169,8 @@ class VectorFieldNet:
         """Parameter initialisation.  NOT flax's RNG-folded lecun_normal (a 'next' row): fan-in
         scaled normals from jax.random-compatible streams; nn_t / nn_xt heads are zero-initialised as
         in the reference (:81,86) unless head_scale > 0."""
-        P = VectorFieldParams(self.dist.dim, self.hidden, self.fourier_random.numel(), self.fourier_random.device)
+        P = VectorFieldParams(self.dist.dim, self.hidden, self.fourier_random.numel(), self.fourier_random.device,
+                              widths=self.widths)
         keys = mrandom.split(rng_key, 8)
         for i, (fi, fo) in enumerate(P.shapes):
             scale = (1.0 / np.sqrt(fi)) * (head_scale if i in (4, 7) else 1.0)
@@ -167,6 +189,8 @@ class VectorFieldNet:
         d.grad_clip = self.grad_clip
         d.ref_mean, d.ref_std = self.ref_mean, self.ref_std
         d.act = self.act
+        if len({w for ws in P.widths for w in ws}) > 1:          # equal widths keep the zero tail: the descriptor of before
+            (d.hidden_t[0], d.hidden_t[1]), (d.hidden_x[0], d.hidden_x[1]), (d.hidden_xt[0], d.hidden_xt[1]) = P.widths
         if self.ref is not None:
             self.ref._fill_ref(d)
         return d
